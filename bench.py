@@ -2,6 +2,7 @@
 """Headline benchmark: GCell/s of a SODA stencil program on B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): jacobi2d, float32, 16384 x 16384,
 iterate 64.  One "step" is one complete run of the program: 64 iterations
@@ -375,6 +376,38 @@ def sharded_parity(rank, world, barrier):
                                   whole.view(torch.int32)).sum().item())}
 
 
+DUMP_CELLS = 1 << 22    # cells --dump-outputs samples in all: <= 32 MB
+
+
+def dump_outputs(directory, library, outputs, regions, row_begin, suffix=''):
+  """--dump-outputs: what the timed path's last step computed, as
+  ``directory/<output name><suffix>.npy``.  Per output, the values (float32,
+  or float64 for other types) of a fixed, seeded sample of the cells of its
+  valid region, in row-major order: the same arguments give the same inputs
+  and the same cells, so two builds compare output for output.  ``regions``
+  are in global coordinates; ``outputs`` hold the global rows
+  ``[row_begin, row_begin + rows)`` and keep the sampled cells among them."""
+  import numpy as np
+  import torch
+  os.makedirs(directory, exist_ok=True)
+  cells = DUMP_CELLS // len(outputs)
+  for (name, _), out, region in zip(library.outputs, outputs, regions):
+    box = [hi - lo for lo, hi in reversed(region)]      # numpy order
+    count = int(np.prod(box))
+    picks = np.arange(count) if count <= cells else np.unique(
+        np.random.default_rng(0).integers(0, count, size=cells))
+    coords = [c + lo for c, (lo, _) in zip(np.unravel_index(picks, box),
+                                           reversed(region))]
+    coords[0] -= row_begin
+    mine = (coords[0] >= 0) & (coords[0] < out.shape[0])
+    flat = np.ravel_multi_index([c[mine] for c in coords], tuple(out.shape))
+    values = out.reshape(-1)[torch.from_numpy(flat).to(out.device)]
+    values = values.cpu().numpy()
+    if values.dtype not in (np.float32, np.float64):
+      values = values.astype(np.float64)
+    np.save(os.path.join(directory, name + suffix + '.npy'), values)
+
+
 def copy_ceiling(world, slab_bytes, reps=3):
   """ms to move `slab_bytes` to each of `world` devices and as many back, both
   directions at once, with plain cudaMemcpyAsync from pinned memory and no
@@ -416,7 +449,16 @@ def main():
   parser.add_argument('--no-cpu-baseline', action='store_true')
   parser.add_argument('--no-extra', action='store_true',
                       help='skip BASELINE configs 3-5 (the `extra` block)')
+  parser.add_argument('--dump-outputs', metavar='DIR',
+                      help='after the timed steps, write a fixed sample of '
+                           'what the last one computed to DIR/<output>.npy')
   args = parser.parse_args()
+  if args.steps < 1:
+    parser.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'b200':
+    parser.error('--dump-outputs dumps the b200 implementation\'s outputs')
+  # the tree may be read-only; nothing is written into it
+  sys.dont_write_bytecode = True
   rank = int(os.environ.get('RANK', '0'))
   world = int(os.environ.get('WORLD_SIZE', '1'))
   if args.impl == 'reference':
@@ -495,10 +537,16 @@ def main():
   start, stop = torch.cuda.Event(True), torch.cuda.Event(True)
   start.record()
   for _ in range(args.steps):
-    step()
+    last = step()
   stop.record()
   barrier()
   clocks = sampler.stop() if sampler else None
+  if args.dump_outputs and distributed:
+    dump_outputs(args.dump_outputs, library, last,
+                 runner.valid_regions(iterate), runner.begin, '.rank%d' % rank)
+  elif args.dump_outputs:
+    dump_outputs(args.dump_outputs, library, [dev_out],
+                 library.valid_regions(dims, iterate), 0)
   ms_total = max_over_ranks(start.elapsed_time(stop))
   ms_per_step = ms_total / args.steps
   value = cells * world * iterate / (ms_per_step * 1e6)     # GCell/s

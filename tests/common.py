@@ -28,6 +28,12 @@ def bench_text(name):
     return handle.read()
 
 
+def golden_output_case(path):
+  """``(program, iterate, dims)`` of ``tests/golden/outputs/<app>_it<N>_<dims>.npz``."""
+  name, it, dims = os.path.basename(path)[:-4].rsplit('_', 2)
+  return name, int(it[2:]), tuple(int(x) for x in dims.split('x'))
+
+
 @functools.lru_cache(maxsize=None)
 def stencil(name, iterate=None):
   return core.Stencil.from_text(bench_text(name), iterate=iterate)

@@ -25,9 +25,7 @@ VECTORS = sorted(glob.glob(os.path.join(common.GOLDEN_DIR, 'outputs',
 
 @pytest.mark.parametrize('path', VECTORS, ids=os.path.basename)
 def test_oracle_reproduces_reference_accepted_outputs(path):
-  name, it, dims = os.path.basename(path)[:-4].rsplit('_', 2)
-  iterate = int(it[2:])
-  dims = tuple(int(x) for x in dims.split('x'))
+  name, iterate, dims = common.golden_output_case(path)
   orc = common.oracle(name, iterate)
   got = orc.run(orc.reference_inputs(dims))
   with np.load(path) as want:

@@ -29,6 +29,19 @@ SANITIZER = shutil.which('compute-sanitizer') or \
     '/usr/local/cuda/bin/compute-sanitizer'
 
 
+def _sanitizer_runs():
+  """An installation may lack the tool or not let this user execute it."""
+  try:
+    return subprocess.run([SANITIZER, '--version'], stdout=subprocess.DEVNULL,
+                          stderr=subprocess.DEVNULL, timeout=120,
+                          check=False).returncode == 0
+  except (OSError, subprocess.SubprocessError):
+    return False
+
+
+SANITIZER_RUNS = _sanitizer_runs()
+
+
 def _run(tool, case, extra=()):
   name, iterate, dims, devices = case
   command = [SANITIZER, '--tool', tool, '--error-exitcode', '86',
@@ -42,8 +55,8 @@ def _run(tool, case, extra=()):
                         timeout=900)
 
 
-@pytest.mark.skipif(not os.path.exists(SANITIZER),
-                    reason='compute-sanitizer not installed')
+@pytest.mark.skipif(not SANITIZER_RUNS,
+                    reason='compute-sanitizer not installed or not executable')
 @pytest.mark.parametrize('case', CASES, ids=['%s-x%d-%s' % c[:3] for c in CASES])
 def test_memcheck_is_clean(case):
   done = _run('memcheck', case)
@@ -52,8 +65,8 @@ def test_memcheck_is_clean(case):
       done.stdout[-3000:]
 
 
-@pytest.mark.skipif(not os.path.exists(SANITIZER),
-                    reason='compute-sanitizer not installed')
+@pytest.mark.skipif(not SANITIZER_RUNS,
+                    reason='compute-sanitizer not installed or not executable')
 @pytest.mark.parametrize('case', CASES[:3],
                          ids=['%s-x%d-%s' % c[:3] for c in CASES[:3]])
 def test_racecheck_is_clean(case):

@@ -58,6 +58,9 @@ def main():
       jobs.append((name, iterate, options))
     for name, iterate, _ in test_parity_gpu.REF_CASES:
       jobs.append((name, iterate, {}))
+    import common
+    for path in test_parity_gpu.REFERENCE_ACCEPTED:
+      jobs.append(common.golden_output_case(path)[:2] + ({},))
     marks = [m for m in
              test_parity_gpu.test_a_run_cut_at_block_boundaries_is_the_same_run
              .pytestmark if m.name == 'parametrize']
