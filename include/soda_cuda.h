@@ -64,12 +64,13 @@ typedef struct soda_cuda_stats_t {
   double kernel_ms;      /* device time of all launches (CUDA events) */
   double h2d_ms;         /* host->device copies, 0 for device buffers */
   double d2h_ms;
-  int64_t cells;         /* prod(dims) */
+  int64_t cells;         /* prod(dims), times the items of a batch */
   int32_t iterate;
   int32_t launches;      /* kernels launched */
   int32_t depth;         /* iterations fused by the main launches */
   int32_t used_tma;      /* 1: TMA input path, 0: plain-load path */
-  int32_t blocks;        /* thread blocks of the last launch */
+  int32_t blocks;        /* thread blocks of the last launch (x * y * z, all
+                            items of a batch) */
   int32_t threads;
   int32_t smem_bytes;
   int32_t reserved;
@@ -148,6 +149,25 @@ int soda_cuda_set_params(const void* const* host_arrays);
  * Inputs are not modified. */
 int soda_cuda_run_device(const void* const* inputs, void* const* outputs,
                          const int32_t* dims, int iterate, void* stream);
+
+/* Batches: `batch` >= 1 independent grids ("items") of the same extents, each
+ * computed exactly as one soda_cuda_run of that item alone would (valid
+ * region and zero border; no item reads another's cells).  Every buffer_t /
+ * pointer describes item 0; items follow at stride prod(extent) elements
+ * (numpy/torch shape (batch, dims[n-1], .., dims[0])).  Param arrays are
+ * shared by all items.
+ * soda_cuda_run_batch: host (copied in and out) or dev (zero copy) buffers,
+ * as soda_cuda_run; params: NULL for programs without params.  Synchronous.
+ * There is no bounds-query mode (such buffers are refused with -12) and no
+ * device list: SODA_CUDA_DEVICES is ignored and the batch runs on the
+ * current device.
+ * soda_cuda_run_device_batch: soda_cuda_run_device on `batch` items.
+ * batch < 1 returns -4 (access_out_of_bounds). */
+int soda_cuda_run_batch(buffer_t* const* inputs, buffer_t* const* outputs,
+                        buffer_t* const* params, int batch);
+int soda_cuda_run_device_batch(const void* const* inputs, void* const* outputs,
+                               const int32_t* dims, int batch, int iterate,
+                               void* stream);
 
 /* One kernel launch: `depth` fused iterations (must be a compiled depth, see
  * soda_cuda_depths) producing streamed planes [row_begin, row_end) of the

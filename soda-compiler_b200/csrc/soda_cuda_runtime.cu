@@ -58,19 +58,21 @@ struct FnInfo {
   int per_sm;
 };
 
-// Rows per block chosen for (kernel, tile grid, rows): the search walks every
-// chunk count, so its answer is kept.
+// Rows per block chosen for (kernel, tile grid, items, rows): the search walks
+// every chunk count, so its answer is kept.
 struct ChunkEntry {
   const void* fn;
   long long grid_x;
+  int batch;
   int rows;
   int chunk_rows;
 };
 
-// A tensor map depends on the address, the extents and the box only.
+// A tensor map depends on the address, the extents (the batch's included) and
+// the box only.
 struct MapEntry {
   const void* ptr;
-  int elem, dim;
+  int elem, dim, batch;
   int32_t dims[kRtMaxDim];
   uint32_t box[kRtMaxDim];
   CUtensorMap map;
@@ -595,11 +597,12 @@ int fn_info(Lane* lane, const ProgramDesc& prog, const KernelVariant* kv,
   return kSuccess;
 }
 
-// Rows per block along the streamed dimension for a launch over `rows` rows.
+// Rows per block along the streamed dimension for a launch over `rows` rows
+// of `batch` items (blockIdx.z).
 int choose_chunk_rows(Lane* lane, const ProgramDesc& prog,
                       const KernelVariant* kv, const void* fn,
-                      const int32_t* dims, int rows, long long* grid_x_out,
-                      int* per_sm_out) {
+                      const int32_t* dims, int rows, int batch,
+                      long long* grid_x_out, int* per_sm_out) {
   int per_sm = 0;
   const int rc = fn_info(lane, prog, kv, fn, &per_sm);
   if (rc != kSuccess) return rc;
@@ -618,48 +621,57 @@ int choose_chunk_rows(Lane* lane, const ProgramDesc& prog,
   {
     std::lock_guard<std::mutex> lock(lane->mutex);
     for (const ChunkEntry& e : lane->chunks)
-      if (e.fn == fn && e.grid_x == grid_x && e.rows == rows)
+      if (e.fn == fn && e.grid_x == grid_x && e.batch == batch &&
+          e.rows == rows)
         return e.chunk_rows;
   }
   const long long resident = static_cast<long long>(per_sm) * lane->sm_count;
-  const int chunks = pick_chunks(grid_x, resident, rows,
+  const int chunks = pick_chunks(grid_x * batch, resident, rows,
                                  kv->lead + kv->out_delay);
   const int chunk_rows = (rows + chunks - 1) / chunks;
   std::lock_guard<std::mutex> lock(lane->mutex);
   if (lane->chunks.size() >= 256) lane->chunks.clear();
-  lane->chunks.push_back({fn, grid_x, rows, chunk_rows});
+  lane->chunks.push_back({fn, grid_x, batch, rows, chunk_rows});
   return chunk_rows;
 }
 
-// The tensor map of input `ptr`, encoded once per (address, shape, box).
-bool tensor_map(Lane* lane, const void* ptr, int elem, int dim,
+// The tensor map of input `ptr`, encoded once per (address, shape, box): rank
+// dim + 1, the outermost dimension counting the `batch` items of the input.
+bool tensor_map(Lane* lane, const void* ptr, int elem, int dim, int batch,
                 const int32_t* dims, const long long* stride,
                 const uint32_t* box, CUtensorMap* out) {
   {
     std::lock_guard<std::mutex> lock(lane->mutex);
     for (const MapEntry& e : lane->maps)
       if (e.ptr == ptr && e.elem == elem && e.dim == dim &&
-          memcmp(e.dims, dims, sizeof(e.dims)) == 0 &&
+          e.batch == batch && memcmp(e.dims, dims, sizeof(e.dims)) == 0 &&
           memcmp(e.box, box, sizeof(e.box)) == 0) {
         *out = e.map;
         return true;
       }
   }
-  cuuint64_t gdim[kRtMaxDim];
+  cuuint64_t gdim[kRtMaxDim + 1];
   cuuint64_t gstride[kRtMaxDim];
-  cuuint32_t estr[kRtMaxDim];
-  cuuint32_t cbox[kRtMaxDim];
+  cuuint32_t estr[kRtMaxDim + 1];
+  cuuint32_t cbox[kRtMaxDim + 1];
+  long long item_stride = 1;
   for (int d = 0; d < dim; ++d) {
     gdim[d] = static_cast<cuuint64_t>(dims[d]);
     estr[d] = 1;
     cbox[d] = box[d];
     if (d > 0) gstride[d - 1] = static_cast<cuuint64_t>(stride[d]) * elem;
+    item_stride *= dims[d];
   }
+  gdim[dim] = static_cast<cuuint64_t>(batch);
+  estr[dim] = 1;
+  cbox[dim] = 1;
+  gstride[dim - 1] = static_cast<cuuint64_t>(item_stride) * elem;
   MapEntry entry;
   memset(&entry, 0, sizeof(entry));
   const CUresult res = g_api.encode(
-      &entry.map, tma_type(elem), dim, const_cast<void*>(ptr), gdim, gstride,
-      cbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+      &entry.map, tma_type(elem), dim + 1, const_cast<void*>(ptr), gdim,
+      gstride, cbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+      CU_TENSOR_MAP_SWIZZLE_NONE,
       CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (res != CUDA_SUCCESS) {
     if (verbose())
@@ -670,6 +682,7 @@ bool tensor_map(Lane* lane, const void* ptr, int elem, int dim,
   entry.ptr = ptr;
   entry.elem = elem;
   entry.dim = dim;
+  entry.batch = batch;
   memcpy(entry.dims, dims, sizeof(entry.dims));
   memcpy(entry.box, box, sizeof(entry.box));
   *out = entry.map;
@@ -704,9 +717,14 @@ int sync_params(Lane* lane, const ProgramDesc& prog) {
   return kSuccess;
 }
 
+// Launches of the variant with `depth` fused iterations over `batch` items
+// of extents `dims` stored one after the other: one launch per kMaxItems
+// items (gridDim.z), all with the same tile and chunk grid.
+constexpr int kMaxItems = 65535;
+
 int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
               const void* const* inputs, void* const* outputs,
-              const int32_t* dims, int row_begin, int row_end,
+              const int32_t* dims, int batch, int row_begin, int row_end,
               const int32_t* valid_lo, const int32_t* valid_hi,
               cudaStream_t stream, int forced_chunk_rows) {
   const KernelVariant* kv = find_variant(prog, depth);
@@ -734,15 +752,17 @@ int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
       args.valid_hi[k][d] = d < prog.dim ? valid_hi[k * kRtMaxDim + d] : 1;
     }
   cells = stride;
-  if (cells >= (1LL << 40)) return kBufferExtentsTooLarge;
+  if (batch < 1) return kAccessOutOfBounds;
+  if (cells * batch >= (1LL << 40)) return kBufferExtentsTooLarge;
   long long tile_blocks = 1;
   for (int d = 0; d < s; ++d) {
     args.tiles[d] = (dims[d] + kv->own[d] - 1) / kv->own[d];
     tile_blocks *= args.tiles[d];
   }
-  if (tile_blocks > 0x7fffffffLL) return kBufferExtentsTooLarge;
+  if (tile_blocks * batch > 0x7fffffffLL) return kBufferExtentsTooLarge;
   args.row_begin = row_begin;
   args.row_end = row_end;
+  args.item_stride = cells;
 
   bool aligned = (dims[0] % kv->vec) == 0;
   bool tma_ok = !env_flag("SODA_CUDA_NO_TMA");   // (tests flip it per call)
@@ -770,37 +790,44 @@ int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
     for (int d = 0; d < prog.dim; ++d)
       box[d] = d == 0 ? kv->box0 : (d < s ? kv->tile[d] : kv->box_rows);
     for (int k = 0; k < prog.n_in && tma_ok; ++k)
-      tma_ok = tensor_map(lane, inputs[k], prog.in_elem[k], prog.dim, dims4,
-                          args.stride, box, &args.in_map[k]);
+      tma_ok = tensor_map(lane, inputs[k], prog.in_elem[k], prog.dim, batch,
+                          dims4, args.stride, box, &args.in_map[k]);
   }
   const void* fn = tma_ok ? kv->kernel_tma : kv->kernel_plain;
   const int rows = row_end - row_begin;
   long long grid_x = 0;
   int per_sm = 0;
-  const int chosen = choose_chunk_rows(lane, prog, kv, fn, dims, rows, &grid_x,
-                                       &per_sm);
+  const int items = std::min(batch, kMaxItems);   // per launch
+  const int chosen = choose_chunk_rows(lane, prog, kv, fn, dims, rows, items,
+                                       &grid_x, &per_sm);
   if (chosen < 0) return chosen;
   args.chunk_rows = forced_chunk_rows > 0 ? std::min(forced_chunk_rows, rows)
                                           : chosen;
   const int chunks = (rows + args.chunk_rows - 1) / args.chunk_rows;
   if (chunks > 65535) return kBufferExtentsTooLarge;
 
-  dim3 grid(static_cast<unsigned>(grid_x), static_cast<unsigned>(chunks));
   dim3 block(kv->threads);
   void* params[] = {&args};
-  SODA_CHECK(cudaLaunchKernel(fn, grid, block, params, kv->smem_bytes, stream),
-             kDeviceRunFailed);
-  lane->stats.launches += 1;
+  for (int begin = 0; begin < batch; begin += kMaxItems) {
+    args.item_begin = begin;
+    dim3 grid(static_cast<unsigned>(grid_x), static_cast<unsigned>(chunks),
+              static_cast<unsigned>(std::min(kMaxItems, batch - begin)));
+    SODA_CHECK(
+        cudaLaunchKernel(fn, grid, block, params, kv->smem_bytes, stream),
+        kDeviceRunFailed);
+    lane->stats.launches += 1;
+  }
   lane->stats.used_tma = tma_ok ? 1 : 0;
-  lane->stats.blocks = static_cast<int32_t>(grid_x * chunks);
+  lane->stats.blocks = static_cast<int32_t>(
+      std::min<long long>(grid_x * chunks * batch, 0x7fffffffLL));
   lane->stats.threads = kv->threads;
   lane->stats.smem_bytes = kv->smem_bytes;
   if (verbose())
     fprintf(stderr,
-            "INFO: %s depth %d on device %d: grid %lld x %d (%d blocks/SM "
-            "resident), %d threads, %d B smem, %s, rows [%d, %d) in chunks "
-            "of %d\n",
-            prog.app_name, depth, lane->ordinal, grid_x, chunks, per_sm,
+            "INFO: %s depth %d on device %d: grid %lld x %d x %d items (%d "
+            "blocks/SM resident), %d threads, %d B smem, %s, rows [%d, %d) in "
+            "chunks of %d\n",
+            prog.app_name, depth, lane->ordinal, grid_x, chunks, batch, per_sm,
             kv->threads, kv->smem_bytes,
             !tma_ok ? "plain loads" : kv->uses_tma ? "TMA" : "128-bit loads",
             row_begin, row_end, args.chunk_rows);
@@ -830,8 +857,8 @@ int chunk_rows(const ProgramDesc& prog, int depth, const int32_t* dims,
   if (rc != kSuccess) return rc;
   const KernelVariant* kv = find_variant(prog, depth);
   if (kv == nullptr || rows < 1) return kInternalError;
-  return choose_chunk_rows(lane, prog, kv, kv->kernel_tma, dims, rows, nullptr,
-                           nullptr);
+  return choose_chunk_rows(lane, prog, kv, kv->kernel_tma, dims, rows, 1,
+                           nullptr, nullptr);
 }
 
 int set_params(const ProgramDesc& prog, const void* const* host_arrays) {
@@ -874,13 +901,14 @@ int launch(const ProgramDesc& prog, int depth, const void* const* inputs,
     g_last_lane = lane;
     g_stats_aggregate = false;
   }
-  return launch_on(lane, prog, depth, inputs, outputs, dims, row_begin,
+  return launch_on(lane, prog, depth, inputs, outputs, dims, 1, row_begin,
                    row_end, valid_lo, valid_hi, stream, forced_chunk_rows);
 }
 
 int run_device(const ProgramDesc& prog, const void* const* inputs,
                void* const* outputs, const int32_t* dims, int iterate,
-               cudaStream_t stream) {
+               cudaStream_t stream, int batch) {
+  if (batch < 1) return kAccessOutOfBounds;
   Lane* lane = nullptr;
   int rc = current_lane(&lane);
   if (rc != kSuccess) return rc;
@@ -895,8 +923,9 @@ int run_device(const ProgramDesc& prog, const void* const* inputs,
   if (rc != kSuccess) return rc;
   const int n_launch = static_cast<int>(depths.size());
 
-  long long cells = 1;
+  long long cells = batch;     // all items
   for (int d = 0; d < prog.dim; ++d) cells *= dims[d];
+  if (cells >= (1LL << 40)) return kBufferExtentsTooLarge;
   // ping-pong between the caller's outputs and one scratch set, arranged so
   // the last launch lands in the outputs
   PoolLease lease(lane);
@@ -920,7 +949,7 @@ int run_device(const ProgramDesc& prog, const void* const* inputs,
     const bool to_outputs = ((n_launch - 1 - l) % 2) == 0;
     for (int k = 0; k < prog.n_out; ++k)
       dst[k] = to_outputs ? outputs[k] : scratch[k];
-    rc = launch_on(lane, prog, depths[l], src, dst, dims, 0,
+    rc = launch_on(lane, prog, depths[l], src, dst, dims, batch, 0,
                    dims[prog.dim - 1], last ? fin.lo : full.lo,
                    last ? fin.hi : full.hi, stream, 0);
     if (rc != kSuccess) return rc;
@@ -1121,7 +1150,7 @@ int run_pipelined(Lane* lane, const ProgramDesc& prog, buffer_t* const* inputs,
       for (int k = 0; k < prog.n_out; ++k)
         dst[k] = to_outputs ? out_dev[k] : scratch[k];
       if (target > frontier[j]) {
-        rc = launch_on(lane, prog, depths[j], src, dst, dims, frontier[j],
+        rc = launch_on(lane, prog, depths[j], src, dst, dims, 1, frontier[j],
                        target, last ? fin.lo : full.lo,
                        last ? fin.hi : full.hi, s_run, 0);
         if (rc != kSuccess) return rc;
@@ -1337,34 +1366,23 @@ int run_sharded(const ProgramDesc& prog, buffer_t* const* inputs,
 
 }  // namespace
 
-int run_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
-                buffer_t* const* outputs, const char* config,
-                buffer_t* const* params) {
+namespace {
+
+int check_present(const ProgramDesc& prog, buffer_t* const* inputs,
+                  buffer_t* const* outputs) {
   for (int k = 0; k < prog.n_in; ++k)
     if (inputs == nullptr || inputs[k] == nullptr) return kBufferArgumentIsNull;
   for (int k = 0; k < prog.n_out; ++k)
     if (outputs == nullptr || outputs[k] == nullptr)
       return kBufferArgumentIsNull;
+  return kSuccess;
+}
 
-  // bounds-query mode (reference host.py:204-252): a buffer with neither host
-  // nor device memory gets its shape filled in; nothing is computed.
-  bool query = false;
-  for (int k = 0; k < prog.n_out; ++k)
-    if (is_query(outputs[k])) {
-      query = true;
-      rewrite(outputs[k], prog.out_elem[k], prog.dim, outputs[k]->min,
-              outputs[k]->extent);
-    }
-  for (int k = 0; k < prog.n_in; ++k)
-    if (is_query(inputs[k])) {
-      query = true;
-      int32_t extent[4] = {0, 0, 0, 0};
-      for (int d = 0; d < prog.dim; ++d)
-        extent[d] = outputs[0]->extent[d] + prog.stencil_dim[d] - 1;
-      rewrite(inputs[k], prog.in_elem[k], prog.dim, outputs[0]->min, extent);
-    }
-  if (query) return kSuccess;
-
+// What every run on buffer_t's checks: element sizes, params (uploaded when
+// given), dense arrays of one common extent, which `dims` receives.
+int check_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
+                  buffer_t* const* outputs, buffer_t* const* params,
+                  int32_t* dims) {
   for (int k = 0; k < prog.n_out; ++k)
     if (outputs[k]->elem_size != prog.out_elem[k]) {
       fprintf(stderr, "ERROR: Buffer %s has type %s but elem_size of the "
@@ -1399,16 +1417,14 @@ int run_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
         if (b->extent[d] != prog.param_size[k][d]) return kAccessOutOfBounds;
       host_arrays[k] = b->host;
     }
-    const int rc_params = set_params(prog, host_arrays);
-    if (rc_params != kSuccess) return rc_params;
+    const int rc = set_params(prog, host_arrays);
+    if (rc != kSuccess) return rc;
   }
 
-  int32_t dims[kRtMaxDim] = {1, 1, 1, 1};
-  long long cells = 1;
+  for (int d = 0; d < kRtMaxDim; ++d) dims[d] = 1;
   for (int d = 0; d < prog.dim; ++d) {
     dims[d] = inputs[0]->extent[d];
     if (dims[d] <= 0) return kAccessOutOfBounds;
-    cells *= dims[d];
   }
   auto dense = [&](const buffer_t* b) {
     int32_t stride = 1;
@@ -1430,11 +1446,111 @@ int run_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
                       "extent\n", prog.out_name[k]);
       return kAccessOutOfBounds;
     }
+  return kSuccess;
+}
 
-  Lane* lane = nullptr;
-  int rc = current_lane(&lane);
+// `batch` items of extents `dims` in each buffer, one after the other: copy
+// the host buffers in, run, copy back, on the default stream.  Device
+// buffers are used in place.
+int run_copied(Lane* lane, const ProgramDesc& prog, buffer_t* const* inputs,
+               buffer_t* const* outputs, const int32_t* dims, int batch) {
+  long long cells = batch;
+  for (int d = 0; d < prog.dim; ++d) cells *= dims[d];
+  cudaStream_t stream = nullptr;
+  PoolLease lease(lane);
+  const void* in_dev[kRtMaxTensors];
+  void* out_dev[kRtMaxTensors];
+  SODA_CHECK(cudaEventRecord(lane->ev[2], stream), kCopyToDeviceFailed);
+  for (int k = 0; k < prog.n_in; ++k) {
+    const size_t bytes = static_cast<size_t>(cells) * prog.in_elem[k];
+    if (inputs[k]->dev != 0) {
+      in_dev[k] = reinterpret_cast<const void*>(inputs[k]->dev);
+      continue;
+    }
+    void* p = lease.get(bytes);
+    if (p == nullptr) return kDeviceMallocFailed;
+    SODA_CHECK(cudaMemcpyAsync(p, inputs[k]->host, bytes,
+                               cudaMemcpyHostToDevice, stream),
+               kCopyToDeviceFailed);
+    in_dev[k] = p;
+  }
+  SODA_CHECK(cudaEventRecord(lane->ev[3], stream), kCopyToDeviceFailed);
+  for (int k = 0; k < prog.n_out; ++k) {
+    const size_t bytes = static_cast<size_t>(cells) * prog.out_elem[k];
+    if (outputs[k]->dev != 0) {
+      out_dev[k] = reinterpret_cast<void*>(outputs[k]->dev);
+      continue;
+    }
+    out_dev[k] = lease.get(bytes);
+    if (out_dev[k] == nullptr) return kDeviceMallocFailed;
+  }
+  const int rc = run_device(prog, in_dev, out_dev, dims, prog.iterate, stream,
+                            batch);
+  if (rc != kSuccess) return rc;
+  SODA_CHECK(cudaEventRecord(lane->ev[4], stream), kCopyToHostFailed);
+  for (int k = 0; k < prog.n_out; ++k) {
+    if (outputs[k]->dev != 0) continue;
+    const size_t bytes = static_cast<size_t>(cells) * prog.out_elem[k];
+    SODA_CHECK(cudaMemcpyAsync(outputs[k]->host, out_dev[k], bytes,
+                               cudaMemcpyDeviceToHost, stream),
+               kCopyToHostFailed);
+  }
+  SODA_CHECK(cudaEventRecord(lane->ev[5], stream), kCopyToHostFailed);
+  SODA_CHECK(cudaStreamSynchronize(stream), kDeviceSyncFailed);
+  lease.completed = true;
+  float ms = 0;
+  if (cudaEventElapsedTime(&ms, lane->ev[2], lane->ev[3]) == cudaSuccess)
+    lane->stats.h2d_ms = ms;
+  if (cudaEventElapsedTime(&ms, lane->ev[4], lane->ev[5]) == cudaSuccess)
+    lane->stats.d2h_ms = ms;
+  const soda_cuda_stats_t* st = last_stats();
+  if (verbose()) {
+    // the two lines the reference host prints (host.py:796-800)
+    fprintf(stderr, "INFO: Kernel execution time: %lf us\n",
+            st->kernel_ms * 1e3);
+    fprintf(stderr, "INFO: Kernel throughput: %lf pixel/ns\n",
+            st->kernel_ms > 0 ? cells / (st->kernel_ms * 1e6) : 0.0);
+  }
+  return kSuccess;
+}
+
+}  // namespace
+
+int run_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
+                buffer_t* const* outputs, const char* config,
+                buffer_t* const* params) {
+  int rc = check_present(prog, inputs, outputs);
   if (rc != kSuccess) return rc;
 
+  // bounds-query mode (reference host.py:204-252): a buffer with neither host
+  // nor device memory gets its shape filled in; nothing is computed.
+  bool query = false;
+  for (int k = 0; k < prog.n_out; ++k)
+    if (is_query(outputs[k])) {
+      query = true;
+      rewrite(outputs[k], prog.out_elem[k], prog.dim, outputs[k]->min,
+              outputs[k]->extent);
+    }
+  for (int k = 0; k < prog.n_in; ++k)
+    if (is_query(inputs[k])) {
+      query = true;
+      int32_t extent[4] = {0, 0, 0, 0};
+      for (int d = 0; d < prog.dim; ++d)
+        extent[d] = outputs[0]->extent[d] + prog.stencil_dim[d] - 1;
+      rewrite(inputs[k], prog.in_elem[k], prog.dim, outputs[0]->min, extent);
+    }
+  if (query) return kSuccess;
+
+  int32_t dims[kRtMaxDim];
+  rc = check_buffers(prog, inputs, outputs, params, dims);
+  if (rc != kSuccess) return rc;
+
+  Lane* lane = nullptr;
+  rc = current_lane(&lane);
+  if (rc != kSuccess) return rc;
+
+  long long cells = 1;
+  for (int d = 0; d < prog.dim; ++d) cells *= dims[d];
   bool all_host = true;
   size_t moved = 0;
   for (int k = 0; k < prog.n_in; ++k) {
@@ -1484,61 +1600,26 @@ int run_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
     return rc;
   }
 
-  cudaStream_t stream = nullptr;
-  PoolLease lease(lane);
-  const void* in_dev[kRtMaxTensors];
-  void* out_dev[kRtMaxTensors];
-  SODA_CHECK(cudaEventRecord(lane->ev[2], stream), kCopyToDeviceFailed);
-  for (int k = 0; k < prog.n_in; ++k) {
-    const size_t bytes = static_cast<size_t>(cells) * prog.in_elem[k];
-    if (inputs[k]->dev != 0) {
-      in_dev[k] = reinterpret_cast<const void*>(inputs[k]->dev);
-      continue;
-    }
-    void* p = lease.get(bytes);
-    if (p == nullptr) return kDeviceMallocFailed;
-    SODA_CHECK(cudaMemcpyAsync(p, inputs[k]->host, bytes,
-                               cudaMemcpyHostToDevice, stream),
-               kCopyToDeviceFailed);
-    in_dev[k] = p;
-  }
-  SODA_CHECK(cudaEventRecord(lane->ev[3], stream), kCopyToDeviceFailed);
-  for (int k = 0; k < prog.n_out; ++k) {
-    const size_t bytes = static_cast<size_t>(cells) * prog.out_elem[k];
-    if (outputs[k]->dev != 0) {
-      out_dev[k] = reinterpret_cast<void*>(outputs[k]->dev);
-      continue;
-    }
-    out_dev[k] = lease.get(bytes);
-    if (out_dev[k] == nullptr) return kDeviceMallocFailed;
-  }
-  rc = run_device(prog, in_dev, out_dev, dims, prog.iterate, stream);
+  return run_copied(lane, prog, inputs, outputs, dims, 1);
+}
+
+int run_batch(const ProgramDesc& prog, buffer_t* const* inputs,
+              buffer_t* const* outputs, buffer_t* const* params, int batch) {
+  if (batch < 1) return kAccessOutOfBounds;
+  int rc = check_present(prog, inputs, outputs);
   if (rc != kSuccess) return rc;
-  SODA_CHECK(cudaEventRecord(lane->ev[4], stream), kCopyToHostFailed);
-  for (int k = 0; k < prog.n_out; ++k) {
-    if (outputs[k]->dev != 0) continue;
-    const size_t bytes = static_cast<size_t>(cells) * prog.out_elem[k];
-    SODA_CHECK(cudaMemcpyAsync(outputs[k]->host, out_dev[k], bytes,
-                               cudaMemcpyDeviceToHost, stream),
-               kCopyToHostFailed);
-  }
-  SODA_CHECK(cudaEventRecord(lane->ev[5], stream), kCopyToHostFailed);
-  SODA_CHECK(cudaStreamSynchronize(stream), kDeviceSyncFailed);
-  lease.completed = true;
-  float ms = 0;
-  if (cudaEventElapsedTime(&ms, lane->ev[2], lane->ev[3]) == cudaSuccess)
-    lane->stats.h2d_ms = ms;
-  if (cudaEventElapsedTime(&ms, lane->ev[4], lane->ev[5]) == cudaSuccess)
-    lane->stats.d2h_ms = ms;
-  const soda_cuda_stats_t* st = last_stats();
-  if (verbose()) {
-    // the two lines the reference host prints (host.py:796-800)
-    fprintf(stderr, "INFO: Kernel execution time: %lf us\n",
-            st->kernel_ms * 1e3);
-    fprintf(stderr, "INFO: Kernel throughput: %lf pixel/ns\n",
-            st->kernel_ms > 0 ? cells / (st->kernel_ms * 1e6) : 0.0);
-  }
-  return kSuccess;
+  for (int k = 0; k < prog.n_in; ++k)
+    if (is_query(inputs[k])) return kBufferArgumentIsNull;
+  for (int k = 0; k < prog.n_out; ++k)
+    if (is_query(outputs[k])) return kBufferArgumentIsNull;
+  int32_t dims[kRtMaxDim];
+  rc = check_buffers(prog, inputs, outputs, params, dims);
+  if (rc != kSuccess) return rc;
+  Lane* lane = nullptr;
+  rc = current_lane(&lane);
+  if (rc != kSuccess) return rc;
+  std::lock_guard<std::mutex> run_lock(lane->run_mutex);
+  return run_copied(lane, prog, inputs, outputs, dims, batch);
 }
 
 int flag_write(void* flag, uint32_t value, cudaStream_t stream) {

@@ -113,11 +113,18 @@ int run_buffers(const ProgramDesc& prog, buffer_t* const* inputs,
 // them.  `run_buffers` calls this when it is given params.
 int set_params(const ProgramDesc& prog, const void* const* host_arrays);
 
-// All `iterate` iterations on device-resident dense arrays, asynchronously on
-// `stream`.  Inputs are not modified.
+// `batch` independent grids of extents `dims` in each buffer (item b starts
+// b * prod(dims) elements in), host or device memory, params as in
+// run_buffers: copied in, run, copied out.  No bounds query (-12) and no
+// device list.
+int run_batch(const ProgramDesc& prog, buffer_t* const* inputs,
+              buffer_t* const* outputs, buffer_t* const* params, int batch);
+
+// All `iterate` iterations on device-resident dense arrays of `batch` items
+// (as in run_batch), asynchronously on `stream`.  Inputs are not modified.
 int run_device(const ProgramDesc& prog, const void* const* inputs,
                void* const* outputs, const int32_t* dims, int iterate,
-               cudaStream_t stream);
+               cudaStream_t stream, int batch = 1);
 
 // One launch of the variant with `depth` fused iterations producing streamed
 // planes [row_begin, row_end) of the outputs; cells of output k outside

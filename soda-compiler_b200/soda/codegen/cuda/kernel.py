@@ -77,6 +77,14 @@ def _log2(n):
   return n.bit_length() - 1
 
 
+def emit_item(p):
+  """The grid item of a batch this block works on, and where it starts in
+  every tensor: plain loads and stores reach it through the per-thread
+  offsets, TMA loads through the item coordinate of the tensor maps."""
+  p.println('const int item = a.item_begin + blockIdx.z;   // of the batch')
+  p.println('const long long item_off = item * a.item_stride;')
+
+
 def _render_stage(stage, ref_code):
   """``Stage.render`` for device code: DSL calls go through the soda_fn_*
   wrappers and let variables get a prefix that cannot clash with the
@@ -129,6 +137,7 @@ def emit_kernel(p, sched):
             sched.lead)
   p.println('const int steps = (r1 - r0) + %d;' %
             (sched.lead + sched.out_delay))
+  emit_item(p)
   p.println()
   p.println('// per-thread vectors: linear position in the plane, where they '
             'land in HBM,')
@@ -156,7 +165,7 @@ def emit_kernel(p, sched):
       p.println('rest /= %d;' % sched.tile[d])
   p.println('(void)rest;')
   p.println('gx[j] = org0 + c0;')
-  p.println('long long off = gx[j];')
+  p.println('long long off = gx[j] + item_off;')
   p.println('bool mine = true;')
   for n in range(len(sched.outputs)):
     p.println('bool ok%d = true;' % n)
@@ -199,7 +208,8 @@ def emit_kernel(p, sched):
     for node in lay.loaded_inputs:
       for b in range(lay.boxes_per_row):
         coords = ['org0 + %d' % (b * lay.box0)] + [
-            'org%d' % d for d in range(1, s)] + ['base + (%s)' % rel_code]
+            'org%d' % d for d in range(1, s)] + ['base + (%s)' % rel_code,
+                                                 'item']
         p.println('soda::tma_load(ring_%s + ((%s) & %d) * %d + %d, '
                   '&a.in_map[%d], bar, %s);' % (
                       node.ident, rel_code, DIN - 1, PLANE, b * lay.box0,

@@ -34,6 +34,7 @@ import collections
 import re
 
 from haoda import util
+from soda.codegen.cuda import kernel as kernel_mod
 from soda.codegen.cuda import plan as plan_mod
 
 _TMA_MAX_BOX = 256
@@ -295,6 +296,7 @@ class _Emitter:
               'the streamed loop' % (sched.lead + sched.out_delay))
     p.println('const int steps = ((r1 - r0) + %d) / %d * %d;' % (
         sched.lead + sched.out_delay + trip - 1, trip, trip))
+    kernel_mod.emit_item(p)
     p.println()
     p.println('// per-thread vectors: position in the plane, offset in HBM, '
               'cells this tile')
@@ -328,7 +330,7 @@ class _Emitter:
         p.println('rest /= %d;' % sched.tile[d])
     p.println('(void)rest;')
     p.println('gx[j] = org0 + c0;')
-    p.println('long long off = gx[j];')
+    p.println('long long off = gx[j] + item_off;')
     p.println('bool mine = true, inside = true;')
     for n in range(len(sched.outputs)):
       p.println('bool ok%d = true;' % n)
@@ -435,7 +437,7 @@ class _Emitter:
         B * sum(lay.row_bytes.values())))
     for node in lay.loaded_inputs:
       p.println('soda::tma_load(queue + %d + ((%s) %% %d) * %d, &a.in_map[%d], '
-                'bar, org0, base + (%s) * %d);' % (
+                'bar, org0, base + (%s) * %d, item);' % (
                     lay.queue_offset[node.index], box_code, G,
                     B * lay.row_bytes[node.index], node.input_index, box_code,
                     B))
@@ -567,7 +569,8 @@ class _Emitter:
     p.println('uint64_t* const bar = &bars[%d];' % slot)
     p.println('soda::mbar_expect_tx(bar, %d);' % sum(lay.plane_bytes.values()))
     for node in lay.loaded_inputs:
-      coords = ['org%d' % d for d in range(s)] + ['base + (%s)' % rel_code]
+      coords = ['org%d' % d for d in range(s)] + ['base + (%s)' % rel_code,
+                                                  'item']
       p.println('soda::tma_load(ring_%s + %d, &a.in_map[%d], bar, %s);' % (
           node.ident, slot * self.PITCH, node.input_index, ', '.join(coords)))
 

@@ -189,6 +189,9 @@ class Library:
         ('soda_cuda_set_params', c_int, [voidpp]),
         ('soda_cuda_run_device', c_int,
          [voidpp, voidpp, i32p, c_int, c_void_p]),
+        ('soda_cuda_run_batch', c_int, [bufpp, bufpp, bufpp, c_int]),
+        ('soda_cuda_run_device_batch', c_int,
+         [voidpp, voidpp, i32p, c_int, c_int, c_void_p]),
         ('soda_cuda_launch', c_int,
          [c_int, voidpp, voidpp, i32p, c_int, c_int, i32p, i32p, c_void_p]),
         ('soda_cuda_launch_chunked', c_int,
@@ -292,8 +295,11 @@ class Library:
     return result
 
   # ---- buffers ----
-  def _describe(self, array, haoda_type, what):
-    """array -> (BufferT, dims); numpy = host memory, torch CUDA = device."""
+  def _describe(self, array, haoda_type, what, batched=False):
+    """array -> (BufferT, dims); numpy = host memory, torch CUDA = device.
+
+    ``batched``: the array holds a batch, shape ``(B, dims[n-1], .., dims[0])``;
+    the buffer describes item 0 and ``dims`` ends with ``B``."""
     elem = util.get_width_in_bytes(haoda_type)
     buf = BufferT()
     if isinstance(array, np.ndarray):
@@ -316,11 +322,13 @@ class Library:
       shape = tuple(array.shape)
     else:
       raise TypeError('%s: expected a numpy array or a torch tensor' % what)
-    if len(shape) != self.dim:
-      raise ValueError('%s must be %d-dimensional' % (what, self.dim))
+    rank = self.dim + (1 if batched else 0)
+    if len(shape) != rank:
+      raise ValueError('%s must be %d-dimensional%s' % (
+          what, rank, ' (a leading batch dimension)' if batched else ''))
     dims = tuple(reversed(shape))
     stride = 1
-    for d, extent in enumerate(dims):
+    for d, extent in enumerate(dims[:self.dim]):
       buf.extent[d], buf.stride[d] = extent, stride
       stride *= extent
     buf.elem_size = elem
@@ -397,26 +405,78 @@ class Library:
       config = ('devices=%s' % (devices if isinstance(devices, str) else
                                 ','.join(str(d) for d in devices))).encode()
     if self.params:
-      arrays = self._param_arrays(params)
-      param_bufs = []
-      for array, (_, haoda_type, size) in zip(arrays, self.params):
-        buf = BufferT()
-        buf.host = array.ctypes.data
-        buf.elem_size = util.get_width_in_bytes(haoda_type)
-        stride = 1
-        for d, extent in enumerate(size):
-          # the reference harness' descriptor of a param (host.py:1022-1030)
-          buf.extent[d], buf.stride[d] = extent, stride
-          stride *= extent
-        param_bufs.append(buf)
-      param_ptrs = (ctypes.POINTER(BufferT) * len(param_bufs))(
-          *[ctypes.pointer(b) for b in param_bufs])
+      param_ptrs, keep_alive = self._param_buffers(params)
       code = self._lib.soda_cuda_run_params(in_ptrs, out_ptrs, param_ptrs,
                                             config)
     else:
       code = self._lib.soda_cuda_run(in_ptrs, out_ptrs, config)
     if code:
       raise CudaError('soda_cuda_run(%s)' % self.app_name, code)
+    return list(outputs)
+
+  def _param_buffers(self, params):
+    """``(buffer_t* array, the arrays it points into)`` of the params."""
+    arrays = self._param_arrays(params)
+    param_bufs = []
+    for array, (_, haoda_type, size) in zip(arrays, self.params):
+      buf = BufferT()
+      buf.host = array.ctypes.data
+      buf.elem_size = util.get_width_in_bytes(haoda_type)
+      stride = 1
+      for d, extent in enumerate(size):
+        # the reference harness' descriptor of a param (host.py:1022-1030)
+        buf.extent[d], buf.stride[d] = extent, stride
+        stride *= extent
+      param_bufs.append(buf)
+    pointers = (ctypes.POINTER(BufferT) * len(param_bufs))(
+        *[ctypes.pointer(b) for b in param_bufs])
+    return pointers, (arrays, param_bufs)
+
+  def run_batch(self, inputs, outputs=None, params=None):
+    """Run the whole program on a batch of independent grids; returns the
+    outputs.
+
+    Every array has shape ``(B, dims[n-1], .., dims[0])``: ``B`` grids of the
+    same extents, each computed exactly as ``run`` computes it alone.  numpy
+    arrays are host memory, torch CUDA tensors are used in place.
+    ``outputs``: arrays to fill, or None to allocate them like the first
+    input.  ``params`` (as for ``run``) are shared by all items.
+    """
+    if len(inputs) != len(self.inputs):
+      raise ValueError('%s takes %d input(s)' % (self.app_name,
+                                                 len(self.inputs)))
+    if outputs is not None and len(outputs) != len(self.outputs):
+      raise ValueError('%s has %d output(s)' % (self.app_name,
+                                                len(self.outputs)))
+    in_bufs, extents = [], None
+    for array, (name, haoda_type) in zip(inputs, self.inputs):
+      buf, got = self._describe(array, haoda_type, 'input `%s`' % name, True)
+      if extents is not None and got != extents:
+        raise ValueError('input `%s` has extent %s (items last), expected %s'
+                         % (name, got, extents))
+      extents = got
+      in_bufs.append(buf)
+    if outputs is None:
+      outputs = [self._allocate_like(inputs[0], haoda_type, extents)
+                 for _, haoda_type in self.outputs]
+    out_bufs = []
+    for array, (name, haoda_type) in zip(outputs, self.outputs):
+      buf, got = self._describe(array, haoda_type, 'output `%s`' % name, True)
+      if got != extents:
+        raise ValueError('output `%s` has extent %s (items last), expected %s'
+                         % (name, got, extents))
+      out_bufs.append(buf)
+    in_ptrs = (ctypes.POINTER(BufferT) * len(in_bufs))(
+        *[ctypes.pointer(b) for b in in_bufs])
+    out_ptrs = (ctypes.POINTER(BufferT) * len(out_bufs))(
+        *[ctypes.pointer(b) for b in out_bufs])
+    param_ptrs = None
+    if self.params:
+      param_ptrs, keep_alive = self._param_buffers(params)
+    code = self._lib.soda_cuda_run_batch(in_ptrs, out_ptrs, param_ptrs,
+                                         extents[-1])
+    if code:
+      raise CudaError('soda_cuda_run_batch(%s)' % self.app_name, code)
     return list(outputs)
 
   @staticmethod
@@ -442,6 +502,16 @@ class Library:
         (ctypes.c_int32 * 4)(*dims), iterate, stream)
     if code:
       raise CudaError('soda_cuda_run_device(%s)' % self.app_name, code)
+
+  def run_device_batch(self, inputs, outputs, dims, batch, iterate=0,
+                       stream=None):
+    """``run_device`` on ``batch`` grids of extents ``dims`` stored one after
+    the other in each array (asynchronous)."""
+    code = self._lib.soda_cuda_run_device_batch(
+        self._pointers(inputs), self._pointers(outputs),
+        (ctypes.c_int32 * 4)(*dims), batch, iterate, stream)
+    if code:
+      raise CudaError('soda_cuda_run_device_batch(%s)' % self.app_name, code)
 
   def ipc_export(self, address):
     """``(handle bytes, offset)`` of the device allocation holding
@@ -594,3 +664,18 @@ def run(stencil, arrays, params=None, devices=None, **kwargs):
     outputs = library.run(inputs, params=params, devices=devices)
     return {name: out for (name, _), out in zip(library.outputs, outputs)}
   return library.run(list(arrays), params=params, devices=devices)
+
+
+def run_batch(stencil, arrays, params=None, **kwargs):
+  """Run ``stencil`` on a batch of independent grids on the current CUDA
+  device: every array has a leading batch dimension (see
+  ``Library.run_batch``).  ``arrays`` and the result take the forms of
+  ``run``."""
+  library = compile_stencil(stencil, **kwargs)
+  if isinstance(arrays, dict):
+    inputs = [arrays[name] for name, _ in library.inputs]
+    if params is None and library.params:
+      params = [arrays[name] for name, _, _ in library.params]
+    outputs = library.run_batch(inputs, params=params)
+    return {name: out for (name, _), out in zip(library.outputs, outputs)}
+  return library.run_batch(list(arrays), params=params)

@@ -109,6 +109,15 @@ def main():
     import test_fullsize_gpu
     for name, iterate, _, _ in test_fullsize_gpu.CONFIGS:
       jobs.append((name, iterate, {}))
+    import test_batch
+    for name, make in test_batch.STENCILS:
+      for style in ('reg', 'ring'):
+        jobs.append((name, make(), {'style': style}))
+    import test_batch_gpu
+    for case in test_batch_gpu.CASES + test_batch_gpu.EXTREME_CASES:
+      kind, name, iterate, _, options, _ = case
+      jobs.append((str(name), test_batch_gpu._stencil(kind, name, iterate),
+                   options))
     # the autotuner test times the planner's own choices, not tuned.json's
     import test_tune_gpu
     marks = [m for m in test_tune_gpu.test_tune_times_every_candidate
