@@ -185,6 +185,12 @@ class _Emitter:
     # writes, where neighbour reads that leave the plane land (see plan)
     self.PITCH = sched.ring_pitch
     self.flat = sched.sdim == 1          # 2-D program: registers only
+    # paired 2-D kernels peel their trips: the steady-state trips, whose rows
+    # every lane stores whole or not at all, are a copy of the trip without
+    # the masked store path; rows are addressed from a pointer per trip
+    self.peel = self.flat and sched.paired
+    assert not self.peel or self.VPT == 1
+    self.steady = False                  # emitting the steady-state trip
     self.DIN = self.lay.in_depth
 
   # ---- naming ---------------------------------------------------------------
@@ -249,11 +255,30 @@ class _Emitter:
     # `steps` is a whole number of trips: the surplus steps compute rows no
     # block stores (beyond mine_hi) from rows that read as 0 or as real data
     trip = lay.box_rows if self.flat else sched.trip
+    if self.peel:
+      self.emit_steady_window(trip)
     if self.flat:
       p.println('for (int i = 0, box = 0; i < steps; i += %d, ++box)' % trip)
     else:
       p.println('for (int i = 0; i < steps; i += %d)' % trip)
     p.do_scope()
+    if self.peel:
+      p.println('for (; static_cast<unsigned>(i - steady_lo) < steady_n; '
+                'i += %d, ++box)' % trip)
+      p.do_scope()
+      self.steady = True
+      self.emit_trip(trip)
+      self.steady = False
+      p.un_scope()
+      p.println('if (i >= steps) break;')
+    self.emit_trip(trip)
+    p.un_scope()
+    p.un_scope()
+    p.println()
+    return lay
+
+  def emit_trip(self, trip):
+    p, sched = self.p, self.sched
     if self.flat:
       self.emit_flat_box()
     for phase in range(trip):
@@ -262,10 +287,37 @@ class _Emitter:
       p.println('const int ii = i + %d;' % phase)
       self.emit_step(phase)
       p.un_scope()
-    p.un_scope()
-    p.un_scope()
+    if self.peel:
+      # the row pointers move to the next trip
+      for node in self.lay.loaded_inputs:
+        p.println('lp%d += pitch * %dll;' % (node.input_index, trip))
+      for node in sched.outputs:
+        p.println('op%d[0] += pitch * %dll;' % (node.output_index, trip))
+
+  def emit_steady_window(self, trip):
+    """Trips ``i`` in [steady_lo, steady_lo + steady_n) store every row of
+    every output with one 128-bit store per lane, or not at all: all their
+    rows lie in each output's valid rows, and no lane of the warp owns only
+    part of its vector or has cells outside the valid columns."""
+    p, sched = self.p, self.sched
+    outs = [node.output_index for node in sched.outputs]
+    p.println('// steady-state trips: the whole trip lies in every output\'s '
+              'valid rows and every lane')
+    p.println('// of the warp stores its whole vector (one 128-bit store) or '
+              'nothing')
+    p.println('const bool whole = own[0] == 0u || (%s);' % ' && '.join(
+        'fast%d[0]' % n for n in outs))
+    lo, hi = 'ok_lo%d' % outs[0], 'ok_lo%d + static_cast<int>(ok_n%d)' % (
+        outs[0], outs[0])
+    for n in outs[1:]:
+      lo = 'max(%s, ok_lo%d)' % (lo, n)
+      hi = 'min(%s, ok_lo%d + static_cast<int>(ok_n%d))' % (hi, n, n)
+    p.println('const int steady_lo = %s;' % lo)
+    p.println('const int steady_hi = %s - %d;' % (hi, trip - 1))
+    p.println('const unsigned steady_n = __all_sync(0xffffffffu, whole) && '
+              'steady_hi > steady_lo ? static_cast<unsigned>(steady_hi - '
+              'steady_lo) : 0u;')
     p.println()
-    return lay
 
   def emit_geometry(self):
     p, sched, s, V, VPT = self.p, self.sched, self.s, self.V, self.VPT
@@ -442,23 +494,33 @@ class _Emitter:
                     B * lay.row_bytes[node.index], node.input_index, box_code,
                     B))
 
-  def flat_plain_load(self, rel_code):
+  def flat_plain_load(self, rel_code, row=None):
     """kTma = false: row ``base + rel`` of every input, cell by cell, into the
-    ``nx_`` registers; cells outside the grid read as 0."""
+    ``nx_`` registers; cells outside the grid read as 0.  Peeled kernels read
+    it ``row`` rows after the trip's row pointer, the others advance the
+    pointer by a row."""
     p, lay, V = self.p, self.lay, self.V
     p.println('const bool lrow_in = static_cast<unsigned>(base + (%s)) < '
               'static_cast<unsigned>(a.dims[%d]);' % (rel_code, self.s))
     for node in lay.loaded_inputs:
       k = node.input_index
+      src = 'lp%d' % k
+      if row:
+        src = '(lp%d + pitch * %dll)' % (k, row)
       p.println('#pragma unroll')
       p.println('for (int k = 0; k < %d; ++k)' % V)
       p.println('  nx_%s[k] = (lrow_in && gx[0] + k >= 0 && gx[0] + k < '
-                'a.dims[0]) ? lp%d[k] : %s(0);' % (node.ident, k, node.c_type))
-      p.println('lp%d += a.stride[%d];' % (k, self.s))
+                'a.dims[0]) ? %s[k] : %s(0);' % (node.ident, src, node.c_type))
+      if row is None:
+        p.println('lp%d += a.stride[%d];' % (k, self.s))
 
   def emit_flat_prologue(self):
     p, lay = self.p, self.lay
     G, B = lay.groups, lay.box_rows
+    if self.peel:
+      p.println('// rows are `pitch` elements apart: dims[0] of a dense 2-D '
+                'grid, an int')
+      p.println('const int pitch = static_cast<int>(a.stride[%d]);' % self.s)
     for node in lay.loaded_inputs:
       p.println('%s nx_%s[%d] = {};   // kTma = false: the next row' % (
           node.c_type, node.ident, self.V))
@@ -486,7 +548,7 @@ class _Emitter:
     p.un_scope()
     p.println('else')
     p.do_scope()
-    self.flat_plain_load('0')
+    self.flat_plain_load('0', 0 if self.peel else None)
     p.un_scope()
     p.println()
 
@@ -538,10 +600,15 @@ class _Emitter:
       else:
         p.println('%s t[%d];' % (node.c_type, V))
         p.println('if (kTma)')
-        p.println('  soda::ld_pack<%s, %d>(t, reinterpret_cast<const %s*>('
-                  'rows_%s + %d));' % (
-                      node.c_type, V, node.c_type, node.ident,
-                      phase * lay.row_bytes[node.index]))
+        if sched.paired:
+          p.println('  for (int k = 0; k < %d; ++k) t[k] = soda::lds_f32('
+                    'rows_%s + %d + 4 * k);' % (
+                        V, node.ident, phase * lay.row_bytes[node.index]))
+        else:
+          p.println('  soda::ld_pack<%s, %d>(t, reinterpret_cast<const %s*>('
+                    'rows_%s + %d));' % (
+                        node.c_type, V, node.c_type, node.ident,
+                        phase * lay.row_bytes[node.index]))
       p.println('else')
       p.do_scope()
       p.println('#pragma unroll')
@@ -559,7 +626,7 @@ class _Emitter:
       p.un_scope()
     p.println('if (!kTma)')
     p.do_scope()
-    self.flat_plain_load('ii + 1')
+    self.flat_plain_load('ii + 1', phase + 1 if self.peel else None)
     p.un_scope()
 
   # ---- 3-D input path: TMA into a shared ring --------------------------------
@@ -717,7 +784,7 @@ class _Emitter:
     skips = (node.output_index is not None and not sched.paired and
              not self.flat and node is sched.stage_nodes[-1] and
              node.hist_oldest is None and node.index not in lay.ring_offset)
-    if node.output_index is not None:
+    if node.output_index is not None and not self.steady:
       n = node.output_index
       p.println('const bool row_ok = static_cast<unsigned>(ii - ok_lo%d) < '
                 'ok_n%d;' % (n, n))
@@ -856,16 +923,24 @@ class _Emitter:
     if node.output_index is not None:
       n = node.output_index
       half = '.v.y' if sched.paired else ''
-      p.println('if (static_cast<unsigned>(ii - ok_lo%d) < fast_n%d[j])' % (
-          n, n))
+      out = 'op%d[j]' % n
+      if self.peel:
+        out = 'orow'
+        p.println('%s* const orow = op%d[j] + pitch * %dll;' % (
+            node.c_type, n, phase))
+      if self.steady:
+        p.println('if (fast%d[j])' % n)
+      else:
+        p.println('if (static_cast<unsigned>(ii - ok_lo%d) < fast_n%d[j])' % (
+            n, n))
       p.do_scope()
       p.println('%s o[%d];' % (node.c_type, V))
       p.println('#pragma unroll')
       p.println('for (int k = 0; k < %d; ++k) o[k] = static_cast<%s>(%s[k]%s);'
                 % (V, node.c_type, target, half))
-      p.println('soda::st_pack_global<%s, %d>(op%d[j], o);' % (
-          node.c_type, V, n))
+      p.println('soda::st_pack_global<%s, %d>(%s, o);' % (node.c_type, V, out))
       p.un_scope()
+    if node.output_index is not None and not self.steady:
       # two-cell vectors: ptxas 12.9 keeps the two `own` bits in predicates and
       # was seen to fold `row_mine && own[j]` into the wrong 3-input LUT
       # (fully owned vectors skipped in two steps of a trip: dbl3d, 64x48
@@ -884,17 +959,17 @@ class _Emitter:
                 '%s(0);' % (node.c_type, target, half, node.c_type))
       p.println('if (own[j] == %du && a.vec_store)' % ((1 << V) - 1))
       p.do_scope()
-      p.println('soda::st_pack_global<%s, %d>(op%d[j], o);' % (
-          node.c_type, V, n))
+      p.println('soda::st_pack_global<%s, %d>(%s, o);' % (node.c_type, V, out))
       p.un_scope()
       p.println('else')
       p.do_scope()
       p.println('#pragma unroll')
       p.println('for (int k = 0; k < %d; ++k)' % V)
-      p.println('  if ((own[j] >> k) & 1u) op%d[j][k] = o[k];' % n)
+      p.println('  if ((own[j] >> k) & 1u) %s[k] = o[k];' % out)
       p.un_scope()
       p.un_scope()
-      p.println('op%d[j] += a.stride[%d];' % (n, s))
+      if not self.peel:
+        p.println('op%d[j] += a.stride[%d];' % (n, s))
     p.un_scope()
     p.un_scope()
 
