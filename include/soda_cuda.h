@@ -169,6 +169,35 @@ int soda_cuda_run_device_batch(const void* const* inputs, void* const* outputs,
                                const int32_t* dims, int batch, int iterate,
                                void* stream);
 
+/* Device-resident arrays of any layout the rule below allows: a tensor view,
+ * rows of a pitched allocation, one channel of a batch, the interior of a
+ * larger array.  Strides are in elements, 5 per tensor (inputs in program
+ * order in `in_strides`, outputs in `out_strides`): stride[0..3] along
+ * dimensions 0..3 (entries >= the program's dim are ignored), then the item
+ * stride (ignored when batch == 1).  For every tensor:
+ *   stride[0] == 1;
+ *   stride[d] >= stride[d-1] * dims[d-1] for 1 <= d < dim;
+ *   batch > 1: item stride >= stride[dim-1] * dims[dim-1];
+ * so no two cells of one tensor share an address.  Transposed, broadcast
+ * (stride 0), negative and overlapping layouts, batch < 1 and empty extents
+ * return -4 (access_out_of_bounds); a tensor spanning 2^48 elements or more,
+ * or 2-D rows 2^31 or more elements apart, -6.  NULL pointers return -12.
+ * These checks come before any device is looked up.  The caller guarantees
+ * that outputs overlap neither the inputs nor each other: this is not
+ * checked.  Cells outside a view read as 0, and nothing outside an output
+ * view is written.  Inputs each of whose strides is a multiple of 16 bytes,
+ * from a 16-byte aligned base, are loaded by TMA; an output whose strides are
+ * multiples of the kernel's vector width, from a 16-byte aligned base, gets
+ * 128-bit stores.  Asynchronous on `stream`, like soda_cuda_run_device.
+ * Out of scope: host arrays, buffer_t strides in soda_cuda_run, broadcast
+ * inputs and multi-device runs. */
+int soda_cuda_run_device_strided(const void* const* inputs,
+                                 const int64_t* in_strides,
+                                 void* const* outputs,
+                                 const int64_t* out_strides,
+                                 const int32_t* dims, int batch, int iterate,
+                                 void* stream);
+
 /* One kernel launch: `depth` fused iterations (must be a compiled depth, see
  * soda_cuda_depths) producing streamed planes [row_begin, row_end) of the
  * outputs from the full input arrays.  `valid_lo` / `valid_hi` hold one box of

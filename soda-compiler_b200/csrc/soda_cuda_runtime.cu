@@ -68,12 +68,13 @@ struct ChunkEntry {
   int chunk_rows;
 };
 
-// A tensor map depends on the address, the extents (the batch's included) and
-// the box only.
+// A tensor map depends on the address, the extents (the batch's included),
+// the strides and the box only.
 struct MapEntry {
   const void* ptr;
   int elem, dim, batch;
   int32_t dims[kRtMaxDim];
+  long long stride[kRtMaxDim + 1];
   uint32_t box[kRtMaxDim];
   CUtensorMap map;
 };
@@ -635,8 +636,10 @@ int choose_chunk_rows(Lane* lane, const ProgramDesc& prog,
   return chunk_rows;
 }
 
-// The tensor map of input `ptr`, encoded once per (address, shape, box): rank
-// dim + 1, the outermost dimension counting the `batch` items of the input.
+// The tensor map of input `ptr` with element strides `stride` (kRtMaxDim + 1
+// entries, the last between items), encoded once per (address, shape,
+// strides, box): rank dim + 1, the outermost dimension counting the `batch`
+// items of the input.
 bool tensor_map(Lane* lane, const void* ptr, int elem, int dim, int batch,
                 const int32_t* dims, const long long* stride,
                 const uint32_t* box, CUtensorMap* out) {
@@ -645,6 +648,7 @@ bool tensor_map(Lane* lane, const void* ptr, int elem, int dim, int batch,
     for (const MapEntry& e : lane->maps)
       if (e.ptr == ptr && e.elem == elem && e.dim == dim &&
           e.batch == batch && memcmp(e.dims, dims, sizeof(e.dims)) == 0 &&
+          memcmp(e.stride, stride, sizeof(e.stride)) == 0 &&
           memcmp(e.box, box, sizeof(e.box)) == 0) {
         *out = e.map;
         return true;
@@ -654,18 +658,16 @@ bool tensor_map(Lane* lane, const void* ptr, int elem, int dim, int batch,
   cuuint64_t gstride[kRtMaxDim];
   cuuint32_t estr[kRtMaxDim + 1];
   cuuint32_t cbox[kRtMaxDim + 1];
-  long long item_stride = 1;
   for (int d = 0; d < dim; ++d) {
     gdim[d] = static_cast<cuuint64_t>(dims[d]);
     estr[d] = 1;
     cbox[d] = box[d];
     if (d > 0) gstride[d - 1] = static_cast<cuuint64_t>(stride[d]) * elem;
-    item_stride *= dims[d];
   }
   gdim[dim] = static_cast<cuuint64_t>(batch);
   estr[dim] = 1;
   cbox[dim] = 1;
-  gstride[dim - 1] = static_cast<cuuint64_t>(item_stride) * elem;
+  gstride[dim - 1] = static_cast<cuuint64_t>(stride[kRtMaxDim]) * elem;
   MapEntry entry;
   memset(&entry, 0, sizeof(entry));
   const CUresult res = g_api.encode(
@@ -684,6 +686,7 @@ bool tensor_map(Lane* lane, const void* ptr, int elem, int dim, int batch,
   entry.dim = dim;
   entry.batch = batch;
   memcpy(entry.dims, dims, sizeof(entry.dims));
+  memcpy(entry.stride, stride, sizeof(entry.stride));
   memcpy(entry.box, box, sizeof(entry.box));
   *out = entry.map;
   std::lock_guard<std::mutex> lock(lane->mutex);
@@ -722,11 +725,50 @@ int sync_params(Lane* lane, const ProgramDesc& prog) {
 // items (gridDim.z), all with the same tile and chunk grid.
 constexpr int kMaxItems = 65535;
 
+// Element strides of every tensor of a launch: [d] along dimension d,
+// [kRtMaxDim] from one item of a batch to the next (check_layout's rule).
+struct Strides {
+  long long in[kRtMaxTensors][kRtMaxDim + 1];
+  long long out[kRtMaxTensors][kRtMaxDim + 1];
+};
+
+// The strides of a dense array of extents `dims`: prod(dims[:d]), items
+// prod(dims) apart.
+void dense_row(const ProgramDesc& prog, const int32_t* dims, long long* row) {
+  long long stride = 1;
+  for (int d = 0; d < kRtMaxDim; ++d) {
+    row[d] = stride;
+    if (d < prog.dim) stride *= dims[d];
+  }
+  row[kRtMaxDim] = stride;
+}
+
+void dense_strides(const ProgramDesc& prog, const int32_t* dims,
+                   Strides* out) {
+  for (int k = 0; k < kRtMaxTensors; ++k) {
+    dense_row(prog, dims, out->in[k]);
+    dense_row(prog, dims, out->out[k]);
+  }
+}
+
+// Is `ptr` 16 B aligned and every stride of the tensor (dimensions 1 .. dim-1
+// and the item stride) a multiple of `multiple` elements?  With the kernel's
+// vector width: whole vectors move with packed accesses.  With 16 B worth of
+// elements: a tensor map can describe the tensor.
+bool strides_aligned(const ProgramDesc& prog, const void* ptr,
+                     const long long* stride, long long multiple) {
+  if (reinterpret_cast<uintptr_t>(ptr) % 16 != 0) return false;
+  for (int d = 1; d < prog.dim; ++d)
+    if (stride[d] % multiple != 0) return false;
+  return stride[kRtMaxDim] % multiple == 0;
+}
+
 int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
               const void* const* inputs, void* const* outputs,
               const int32_t* dims, int batch, int row_begin, int row_end,
               const int32_t* valid_lo, const int32_t* valid_hi,
-              cudaStream_t stream, int forced_chunk_rows) {
+              cudaStream_t stream, int forced_chunk_rows,
+              const Strides& strides) {
   const KernelVariant* kv = find_variant(prog, depth);
   if (kv == nullptr) {
     fprintf(stderr, "ERROR: %s was not compiled with temporal depth %d\n",
@@ -738,12 +780,11 @@ int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
 
   StreamArgs args;
   memset(&args, 0, sizeof(args));
-  long long stride = 1, cells = 1;
+  long long cells = 1;
   int32_t dims4[kRtMaxDim];
   for (int d = 0; d < kRtMaxDim; ++d) {
     dims4[d] = args.dims[d] = d < prog.dim ? dims[d] : 1;
-    args.stride[d] = stride;
-    stride *= args.dims[d];
+    cells *= args.dims[d];
     args.tiles[d] = 1;
   }
   for (int k = 0; k < prog.n_out; ++k)
@@ -751,7 +792,6 @@ int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
       args.valid_lo[k][d] = d < prog.dim ? valid_lo[k * kRtMaxDim + d] : 0;
       args.valid_hi[k][d] = d < prog.dim ? valid_hi[k * kRtMaxDim + d] : 1;
     }
-  cells = stride;
   if (batch < 1) return kAccessOutOfBounds;
   if (cells * batch >= (1LL << 40)) return kBufferExtentsTooLarge;
   long long tile_blocks = 1;
@@ -762,22 +802,27 @@ int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
   if (tile_blocks * batch > 0x7fffffffLL) return kBufferExtentsTooLarge;
   args.row_begin = row_begin;
   args.row_end = row_end;
-  args.item_stride = cells;
 
-  bool aligned = (dims[0] % kv->vec) == 0;
+  // Per tensor: whole vectors move with packed accesses when its base and
+  // strides keep them aligned; the TMA path needs every input to be
+  // describable by a tensor map (16 B aligned base and byte strides).
   bool tma_ok = !env_flag("SODA_CUDA_NO_TMA");   // (tests flip it per call)
   for (int k = 0; k < prog.n_in; ++k) {
     args.in_ptr[k] = inputs[k];
-    const uintptr_t p = reinterpret_cast<uintptr_t>(inputs[k]);
-    if (p % 16 != 0) aligned = tma_ok = false;
-    if ((static_cast<long long>(dims[0]) * prog.in_elem[k]) % 16 != 0)
+    memcpy(args.in_stride[k], strides.in[k], sizeof(args.in_stride[k]));
+    args.vec_load[k] =
+        strides_aligned(prog, inputs[k], strides.in[k], kv->vec) ? 1 : 0;
+    // (elements are 1, 2, 4 or 8 bytes: 16 B is a whole number of them)
+    const long long cells_16b = 16 / prog.in_elem[k];
+    if (!strides_aligned(prog, inputs[k], strides.in[k], cells_16b))
       tma_ok = false;
   }
   for (int k = 0; k < prog.n_out; ++k) {
     args.out_ptr[k] = outputs[k];
-    if (reinterpret_cast<uintptr_t>(outputs[k]) % 16 != 0) aligned = false;
+    memcpy(args.out_stride[k], strides.out[k], sizeof(args.out_stride[k]));
+    args.vec_store[k] =
+        strides_aligned(prog, outputs[k], strides.out[k], kv->vec) ? 1 : 0;
   }
-  args.vec_store = aligned ? 1 : 0;
   if (prog.n_param > 0) {
     const int rc = sync_params(lane, prog);
     if (rc != kSuccess) return rc;
@@ -791,7 +836,7 @@ int launch_on(Lane* lane, const ProgramDesc& prog, int depth,
       box[d] = d == 0 ? kv->box0 : (d < s ? kv->tile[d] : kv->box_rows);
     for (int k = 0; k < prog.n_in && tma_ok; ++k)
       tma_ok = tensor_map(lane, inputs[k], prog.in_elem[k], prog.dim, batch,
-                          dims4, args.stride, box, &args.in_map[k]);
+                          dims4, strides.in[k], box, &args.in_map[k]);
   }
   const void* fn = tma_ok ? kv->kernel_tma : kv->kernel_plain;
   const int rows = row_end - row_begin;
@@ -901,14 +946,20 @@ int launch(const ProgramDesc& prog, int depth, const void* const* inputs,
     g_last_lane = lane;
     g_stats_aggregate = false;
   }
+  Strides dense;
+  dense_strides(prog, dims, &dense);
   return launch_on(lane, prog, depth, inputs, outputs, dims, 1, row_begin,
-                   row_end, valid_lo, valid_hi, stream, forced_chunk_rows);
+                   row_end, valid_lo, valid_hi, stream, forced_chunk_rows,
+                   dense);
 }
 
-int run_device(const ProgramDesc& prog, const void* const* inputs,
+namespace {
+
+// All `iterate` iterations on device arrays of `batch` items whose layout
+// `caller` gives (the caller's inputs and outputs; scratch is dense).
+int run_layout(const ProgramDesc& prog, const void* const* inputs,
                void* const* outputs, const int32_t* dims, int iterate,
-               cudaStream_t stream, int batch) {
-  if (batch < 1) return kAccessOutOfBounds;
+               cudaStream_t stream, int batch, const Strides& caller) {
   Lane* lane = nullptr;
   int rc = current_lane(&lane);
   if (rc != kSuccess) return rc;
@@ -943,18 +994,32 @@ int run_device(const ProgramDesc& prog, const void* const* inputs,
   SODA_CHECK(cudaEventRecord(lane->ev[0], stream), kDeviceRunFailed);
   const void* src[kRtMaxTensors];
   void* dst[kRtMaxTensors];
+  // each launch gets the strides of the arrays it reads and writes: the
+  // caller's, or the dense ones of the scratch set
+  long long dense[kRtMaxDim + 1];
+  dense_row(prog, dims, dense);
+  Strides strides = caller;
+  bool all_tma = true;    // the stats say TMA only if every launch used it
   for (int k = 0; k < prog.n_in; ++k) src[k] = inputs[k];
   for (int l = 0; l < n_launch; ++l) {
     const bool last = l + 1 == n_launch;
     const bool to_outputs = ((n_launch - 1 - l) % 2) == 0;
-    for (int k = 0; k < prog.n_out; ++k)
+    for (int k = 0; k < prog.n_out; ++k) {
       dst[k] = to_outputs ? outputs[k] : scratch[k];
+      memcpy(strides.out[k], to_outputs ? caller.out[k] : dense,
+             sizeof(dense));
+    }
     rc = launch_on(lane, prog, depths[l], src, dst, dims, batch, 0,
                    dims[prog.dim - 1], last ? fin.lo : full.lo,
-                   last ? fin.hi : full.hi, stream, 0);
+                   last ? fin.hi : full.hi, stream, 0, strides);
     if (rc != kSuccess) return rc;
-    for (int k = 0; k < prog.n_out; ++k) src[k] = dst[k];
+    all_tma = all_tma && lane->stats.used_tma;
+    for (int k = 0; k < prog.n_out; ++k) {
+      src[k] = dst[k];
+      memcpy(strides.in[k], strides.out[k], sizeof(dense));
+    }
   }
+  lane->stats.used_tma = all_tma ? 1 : 0;
   SODA_CHECK(cudaEventRecord(lane->ev[1], stream), kDeviceRunFailed);
   if (n_launch > 1) {
     // scratch goes back to the pool when the stream has drained past here
@@ -962,6 +1027,94 @@ int run_device(const ProgramDesc& prog, const void* const* inputs,
   }
   lease.completed = true;
   return kSuccess;
+}
+
+// check_layout for one tensor: 0, or the code that refuses it.
+int check_tensor_layout(const ProgramDesc& prog, const int32_t* dims,
+                        int batch, const int64_t* stride) {
+  const int last = prog.dim - 1;
+  if (stride[0] != 1) return kAccessOutOfBounds;
+  // stride[d] >= stride[d-1] * dims[d-1], without overflow (all positive)
+  for (int d = 1; d < prog.dim; ++d)
+    if (stride[d] < 1 || stride[d] / dims[d - 1] < stride[d - 1])
+      return kAccessOutOfBounds;
+  const int64_t item = stride[kRtMaxDim];
+  if (batch > 1 && (item < 1 || item / dims[last] < stride[last]))
+    return kAccessOutOfBounds;
+  // what one tensor spans stays far from overflowing 64-bit offsets, and 2-D
+  // rows are less than 2^31 elements apart (the kernels' row pitch)
+  const int64_t outer = batch > 1 ? item : stride[last];
+  const int64_t count = batch > 1 ? batch : dims[last];
+  if (outer > (int64_t(1) << 48) / count) return kBufferExtentsTooLarge;
+  if (prog.dim == 2 && stride[1] > 0x7fffffffLL) return kBufferExtentsTooLarge;
+  return kSuccess;
+}
+
+}  // namespace
+
+int check_layout(const ProgramDesc& prog, const int32_t* dims, int batch,
+                 const int64_t* in_strides, const int64_t* out_strides) {
+  if (batch < 1) return kAccessOutOfBounds;
+  for (int d = 0; d < prog.dim; ++d)
+    if (dims[d] < 1) return kAccessOutOfBounds;
+  for (int k = 0; k < prog.n_in; ++k) {
+    const int rc = check_tensor_layout(prog, dims, batch,
+                                       in_strides + k * (kRtMaxDim + 1));
+    if (rc != kSuccess) return rc;
+  }
+  for (int k = 0; k < prog.n_out; ++k) {
+    const int rc = check_tensor_layout(prog, dims, batch,
+                                       out_strides + k * (kRtMaxDim + 1));
+    if (rc != kSuccess) return rc;
+  }
+  return kSuccess;
+}
+
+int run_device(const ProgramDesc& prog, const void* const* inputs,
+               void* const* outputs, const int32_t* dims, int iterate,
+               cudaStream_t stream, int batch) {
+  if (batch < 1) return kAccessOutOfBounds;
+  Strides dense;
+  dense_strides(prog, dims, &dense);
+  return run_layout(prog, inputs, outputs, dims, iterate, stream, batch,
+                    dense);
+}
+
+int run_device_strided(const ProgramDesc& prog, const void* const* inputs,
+                       const int64_t* in_strides, void* const* outputs,
+                       const int64_t* out_strides, const int32_t* dims,
+                       int batch, int iterate, cudaStream_t stream) {
+  if (inputs == nullptr || outputs == nullptr || in_strides == nullptr ||
+      out_strides == nullptr || dims == nullptr)
+    return kBufferArgumentIsNull;
+  for (int k = 0; k < prog.n_in; ++k)
+    if (inputs[k] == nullptr) return kBufferArgumentIsNull;
+  for (int k = 0; k < prog.n_out; ++k)
+    if (outputs[k] == nullptr) return kBufferArgumentIsNull;
+  const int rc = check_layout(prog, dims, batch, in_strides, out_strides);
+  if (rc != kSuccess) {
+    fprintf(stderr, "ERROR: %s: array layout refused (%d): strides must be "
+                    "1, then at least the span of the previous dimension, "
+                    "items beyond the last\n", prog.app_name, rc);
+    return rc;
+  }
+  // entries past the program's rank are not the caller's to give; a single
+  // item's item stride is its span
+  Strides strides;
+  auto take = [&](const int64_t* given, long long* row) {
+    for (int d = 0; d <= kRtMaxDim; ++d)
+      row[d] = d < prog.dim ? given[d] : 0;
+    row[kRtMaxDim] = batch > 1 ? given[kRtMaxDim]
+                               : given[prog.dim - 1] * dims[prog.dim - 1];
+  };
+  for (int k = 0; k < kRtMaxTensors; ++k) {
+    take(k < prog.n_in ? in_strides + k * (kRtMaxDim + 1) : in_strides,
+         strides.in[k]);
+    take(k < prog.n_out ? out_strides + k * (kRtMaxDim + 1) : out_strides,
+         strides.out[k]);
+  }
+  return run_layout(prog, inputs, outputs, dims, iterate, stream, batch,
+                    strides);
 }
 
 namespace {
@@ -1087,6 +1240,8 @@ int run_pipelined(Lane* lane, const ProgramDesc& prog, buffer_t* const* inputs,
     hi = std::min(std::max(0, hi - slab.local_begin), rows);
   }
 
+  Strides dense;
+  dense_strides(prog, dims, &dense);
   std::vector<int> frontier(need_lo);
   SODA_CHECK(cudaEventRecord(lane->ev[2], s_in), kCopyToDeviceFailed);
   SODA_CHECK(cudaEventRecord(lane->ev[0], s_run), kDeviceRunFailed);
@@ -1152,7 +1307,7 @@ int run_pipelined(Lane* lane, const ProgramDesc& prog, buffer_t* const* inputs,
       if (target > frontier[j]) {
         rc = launch_on(lane, prog, depths[j], src, dst, dims, 1, frontier[j],
                        target, last ? fin.lo : full.lo,
-                       last ? fin.hi : full.hi, s_run, 0);
+                       last ? fin.hi : full.hi, s_run, 0, dense);
         if (rc != kSuccess) return rc;
         frontier[j] = target;
       }

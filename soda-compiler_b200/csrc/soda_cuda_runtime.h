@@ -126,6 +126,25 @@ int run_device(const ProgramDesc& prog, const void* const* inputs,
                void* const* outputs, const int32_t* dims, int iterate,
                cudaStream_t stream, int batch = 1);
 
+// run_device on arrays of any layout check_layout accepts: kRtMaxDim + 1
+// element strides per tensor (along dimensions 0 .. dim-1, entries beyond
+// ignored, then the item stride, ignored when batch == 1).  NULL pointers give
+// -12 and refused layouts -4 / -6, both before any device is looked up.
+// Outputs must not overlap the inputs or each other (not checked).
+int run_device_strided(const ProgramDesc& prog, const void* const* inputs,
+                       const int64_t* in_strides, void* const* outputs,
+                       const int64_t* out_strides, const int32_t* dims,
+                       int batch, int iterate, cudaStream_t stream);
+
+// The layouts the kernels address, where no two cells of a tensor share an
+// address: stride[0] == 1, stride[d] >= stride[d-1] * dims[d-1], and for
+// batch > 1 item stride >= stride[dim-1] * dims[dim-1].  Anything else
+// (transposed, broadcast, negative, overlapping), batch < 1 and empty extents
+// give -4; a tensor spanning 2^48 elements or more, or 2-D rows 2^31 or more
+// elements apart, -6.  Needs no device.
+int check_layout(const ProgramDesc& prog, const int32_t* dims, int batch,
+                 const int64_t* in_strides, const int64_t* out_strides);
+
 // One launch of the variant with `depth` fused iterations producing streamed
 // planes [row_begin, row_end) of the outputs; cells of output k outside
 // [valid_lo[4k..], valid_hi[4k..]) are stored as 0 (one box of kRtMaxDim ints

@@ -78,11 +78,38 @@ def _log2(n):
 
 
 def emit_item(p):
-  """The grid item of a batch this block works on, and where it starts in
-  every tensor: plain loads and stores reach it through the per-thread
-  offsets, TMA loads through the item coordinate of the tensor maps."""
+  """The grid item of a batch this block works on: plain loads and stores
+  reach it through the per-tensor offsets (``emit_offsets``), TMA loads
+  through the item coordinate of the tensor maps."""
   p.println('const int item = a.item_begin + blockIdx.z;   // of the batch')
-  p.println('const long long item_off = item * a.item_stride;')
+
+
+def emit_offset_arrays(p, inputs, outputs, vpt):
+  """Declare the per-thread HBM offsets of every loaded input and output."""
+  for node in inputs:
+    p.println('long long ioff%d[%d];   // input %d' % (
+        node.input_index, vpt, node.input_index))
+  for node in outputs:
+    p.println('long long ooff%d[%d];   // output %d' % (
+        node.output_index, vpt, node.output_index))
+
+
+def emit_offsets(p, inputs, outputs, sdim):
+  """Inside the per-vector loop over ``j``: where vector ``j`` of the item
+  lies in each tensor, in elements from its base, for plane 0 of the streamed
+  dimension.  Every tensor has strides of its own (a view, a pitched
+  allocation); in the TMA instance the inputs' offsets are dead code."""
+  def offset(which, k):
+    terms = ['gx[j]', 'item * a.%s_stride[%d][soda::kMaxDim]' % (which, k)]
+    terms += ['gc%d[j] * a.%s_stride[%d][%d]' % (d, which, k, d)
+              for d in range(1, sdim)]
+    return ' + '.join(terms)
+  for node in inputs:
+    p.println('ioff%d[j] = %s;' % (node.input_index,
+                                   offset('in', node.input_index)))
+  for node in outputs:
+    p.println('ooff%d[j] = %s;' % (node.output_index,
+                                   offset('out', node.output_index)))
 
 
 def _render_stage(stage, ref_code):
@@ -144,7 +171,7 @@ def emit_kernel(p, sched):
   p.println('// which cells this tile owns (store) and which are in the '
             'valid region (else 0)')
   p.println('int pos[%d];' % VPT)
-  p.println('long long goff[%d];' % VPT)
+  emit_offset_arrays(p, lay.loaded_inputs, sched.outputs, VPT)
   p.println('unsigned own[%d];' % VPT)
   for n in range(len(sched.outputs)):
     p.println('unsigned val%d[%d];   // output %d: cells in ITS valid region' %
@@ -165,20 +192,18 @@ def emit_kernel(p, sched):
       p.println('rest /= %d;' % sched.tile[d])
   p.println('(void)rest;')
   p.println('gx[j] = org0 + c0;')
-  p.println('long long off = gx[j] + item_off;')
   p.println('bool mine = true;')
   for n in range(len(sched.outputs)):
     p.println('bool ok%d = true;' % n)
   for d in range(1, s):
     p.println('gc%d[j] = org%d + c%d;' % (d, d, d))
-    p.println('off += gc%d[j] * a.stride[%d];' % (d, d))
     p.println('mine = mine && c%d >= %d && c%d < %d && gc%d[j] < a.dims[%d];' %
               (d, sched.tile_halo_lo[d], d,
                sched.tile[d] - sched.tile_halo_hi[d], d, d))
     for n in range(len(sched.outputs)):
       p.println('ok%d = ok%d && gc%d[j] >= a.valid_lo[%d][%d] && gc%d[j] < '
                 'a.valid_hi[%d][%d];' % (n, n, d, n, d, d, n, d))
-  p.println('goff[j] = off;')
+  emit_offsets(p, lay.loaded_inputs, sched.outputs, s)
   p.println('unsigned m = 0;')
   for n in range(len(sched.outputs)):
     p.println('unsigned v%d = 0;' % n)
@@ -228,11 +253,12 @@ def emit_kernel(p, sched):
           'gc%d[j] >= 0 && gc%d[j] < a.dims[%d]' % (d, d, d)
           for d in range(1, s)])
       p.println('const bool in = %s;' % cond)
+      k = node.input_index
       p.println('const %s* src = static_cast<const %s*>(a.in_ptr[%d]) + '
-                'lrow * a.stride[%d] + goff[j];' % (
-                    node.c_type, node.c_type, node.input_index, s))
-      p.println('if (in && a.vec_store && gx[j] >= 0 && gx[j] + %d <= '
-                'a.dims[0])' % V)
+                'lrow * a.in_stride[%d][%d] + ioff%d[j];' % (
+                    node.c_type, node.c_type, k, k, s, k))
+      p.println('if (in && a.vec_load[%d] && gx[j] >= 0 && gx[j] + %d <= '
+                'a.dims[0])' % (k, V))
       p.do_scope()
       p.println('soda::ld_pack<%s, %d>(t, src);' % (node.c_type, V))
       p.un_scope()
@@ -380,9 +406,10 @@ def _emit_stage(p, sched, lay, node):
     full = (1 << V) - 1
     p.println('if (row_mine && own[j])')
     p.do_scope()
+    n = node.output_index
     p.println('%s* const dst = static_cast<%s*>(a.out_ptr[%d]) + row * '
-              'a.stride[%d] + goff[j];' % (node.c_type, node.c_type,
-                                           node.output_index, s))
+              'a.out_stride[%d][%d] + ooff%d[j];' % (node.c_type, node.c_type,
+                                                     n, n, s, n))
     p.println('const unsigned keep = row_ok ? val%d[j] : 0u;' % node.output_index)
     p.println('if (keep != %du)' % full)
     p.do_scope()
@@ -390,7 +417,7 @@ def _emit_stage(p, sched, lay, node):
     p.println('for (int k = 0; k < %d; ++k)' % V)
     p.println('  if (!((keep >> k) & 1u)) r[k] = %s(0);' % node.c_type)
     p.un_scope()
-    p.println('if (own[j] == %du && a.vec_store)' % full)
+    p.println('if (own[j] == %du && a.vec_store[%d])' % (full, n))
     p.do_scope()
     p.println('soda::st_pack_global<%s, %d>(dst, r);' % (node.c_type, V))
     p.un_scope()

@@ -290,9 +290,11 @@ class _Emitter:
     if self.peel:
       # the row pointers move to the next trip
       for node in self.lay.loaded_inputs:
-        p.println('lp%d += pitch * %dll;' % (node.input_index, trip))
+        p.println('lp%d += ipitch%d * %dll;' % (node.input_index,
+                                              node.input_index, trip))
       for node in sched.outputs:
-        p.println('op%d[0] += pitch * %dll;' % (node.output_index, trip))
+        p.println('op%d[0] += opitch%d * %dll;' % (node.output_index,
+                                                 node.output_index, trip))
 
   def emit_steady_window(self, trip):
     """Trips ``i`` in [steady_lo, steady_lo + steady_n) store every row of
@@ -354,7 +356,8 @@ class _Emitter:
               'cells this tile')
     p.println('// owns (store) and cells in the valid region (else 0)')
     p.println('int pos[%d];' % VPT)
-    p.println('long long goff[%d];' % VPT)
+    kernel_mod.emit_offset_arrays(p, self.lay.loaded_inputs, sched.outputs,
+                                  VPT)
     p.println('unsigned own[%d];' % VPT)
     for n in range(len(sched.outputs)):
       p.println('unsigned val%d[%d];   // output %d: cells in ITS valid region'
@@ -382,13 +385,11 @@ class _Emitter:
         p.println('rest /= %d;' % sched.tile[d])
     p.println('(void)rest;')
     p.println('gx[j] = org0 + c0;')
-    p.println('long long off = gx[j] + item_off;')
     p.println('bool mine = true, inside = true;')
     for n in range(len(sched.outputs)):
       p.println('bool ok%d = true;' % n)
     for d in range(1, s):
       p.println('gc%d[j] = org%d + c%d;' % (d, d, d))
-      p.println('off += gc%d[j] * a.stride[%d];' % (d, d))
       p.println('mine = mine && c%d >= %d && c%d < %d && gc%d[j] < a.dims[%d];'
                 % (d, sched.tile_halo_lo[d], d,
                    sched.tile[d] - sched.tile_halo_hi[d], d, d))
@@ -397,7 +398,7 @@ class _Emitter:
                   'a.valid_hi[%d][%d];' % (n, n, d, n, d, d, n, d))
       p.println('inside = inside && gc%d[j] >= 0 && gc%d[j] < a.dims[%d];' % (
           d, d, d))
-    p.println('goff[j] = off;')
+    kernel_mod.emit_offsets(p, self.lay.loaded_inputs, sched.outputs, s)
     p.println('xin[j] = inside && gx[j] >= 0 && gx[j] + %d <= a.dims[0];' % V)
     p.println('unsigned m = 0;')
     for n in range(len(sched.outputs)):
@@ -416,8 +417,8 @@ class _Emitter:
     p.println('own[j] = m;')
     for n in range(len(sched.outputs)):
       p.println('val%d[j] = v%d;' % (n, n))
-      p.println('fast%d[j] = m == %du && v%d == %du && a.vec_store;' % (
-          n, (1 << V) - 1, n, (1 << V) - 1))
+      p.println('fast%d[j] = m == %du && v%d == %du && a.vec_store[%d];' % (
+          n, (1 << V) - 1, n, (1 << V) - 1, n))
     p.un_scope()
     p.println()
 
@@ -459,7 +460,8 @@ class _Emitter:
       p.println('#pragma unroll')
       p.println('for (int j = 0; j < %d; ++j)' % self.VPT)
       p.println('  op%d[j] = static_cast<%s*>(a.out_ptr[%d]) + (base - %d) * '
-                'a.stride[%d] + goff[j];' % (n, node.c_type, n, lag, s))
+                'a.out_stride[%d][%d] + ooff%d[j];' % (n, node.c_type, n, lag,
+                                                       n, s, n))
     p.println()
 
   def emit_histories(self):
@@ -506,28 +508,34 @@ class _Emitter:
       k = node.input_index
       src = 'lp%d' % k
       if row:
-        src = '(lp%d + pitch * %dll)' % (k, row)
+        src = '(lp%d + ipitch%d * %dll)' % (k, k, row)
       p.println('#pragma unroll')
       p.println('for (int k = 0; k < %d; ++k)' % V)
       p.println('  nx_%s[k] = (lrow_in && gx[0] + k >= 0 && gx[0] + k < '
                 'a.dims[0]) ? %s[k] : %s(0);' % (node.ident, src, node.c_type))
       if row is None:
-        p.println('lp%d += a.stride[%d];' % (k, self.s))
+        p.println('lp%d += a.in_stride[%d][%d];' % (k, k, self.s))
 
   def emit_flat_prologue(self):
     p, lay = self.p, self.lay
     G, B = lay.groups, lay.box_rows
     if self.peel:
-      p.println('// rows are `pitch` elements apart: dims[0] of a dense 2-D '
-                'grid, an int')
-      p.println('const int pitch = static_cast<int>(a.stride[%d]);' % self.s)
+      p.println('// rows of each tensor are its `pitch` elements apart (the '
+                'runtime keeps 2-D row')
+      p.println('// strides below 2^31)')
+      for node in lay.loaded_inputs:
+        p.println('const int ipitch%d = static_cast<int>(a.in_stride[%d][%d]);'
+                  % (node.input_index, node.input_index, self.s))
+      for node in self.sched.outputs:
+        p.println('const int opitch%d = static_cast<int>(a.out_stride[%d][%d]);'
+                  % (node.output_index, node.output_index, self.s))
     for node in lay.loaded_inputs:
+      k = node.input_index
       p.println('%s nx_%s[%d] = {};   // kTma = false: the next row' % (
           node.c_type, node.ident, self.V))
       p.println('const %s* lp%d = static_cast<const %s*>(a.in_ptr[%d]) + '
-                'base * a.stride[%d] + goff[0];' % (
-                    node.c_type, node.input_index, node.c_type,
-                    node.input_index, self.s))
+                'base * a.in_stride[%d][%d] + ioff%d[0];' % (
+                    node.c_type, k, node.c_type, k, k, self.s, k))
     p.println('if (kTma)')
     p.do_scope()
     p.println('if (lane == 0)')
@@ -654,11 +662,12 @@ class _Emitter:
           'gc%d[j] >= 0 && gc%d[j] < a.dims[%d]' % (d, d, d)
           for d in range(1, s)])
       p.println('const bool in = %s;' % cond)
+      k = node.input_index
       p.println('const %s* src = static_cast<const %s*>(a.in_ptr[%d]) + '
-                'lrow * a.stride[%d] + goff[j];' % (
-                    node.c_type, node.c_type, node.input_index, s))
-      p.println('if (in && a.vec_store && gx[j] >= 0 && gx[j] + %d <= '
-                'a.dims[0])' % V)
+                'lrow * a.in_stride[%d][%d] + ioff%d[j];' % (
+                    node.c_type, node.c_type, k, k, s, k))
+      p.println('if (in && a.vec_load[%d] && gx[j] >= 0 && gx[j] + %d <= '
+                'a.dims[0])' % (k, V))
       p.do_scope()
       p.println('soda::ld_pack<%s, %d>(t, src);' % (node.c_type, V))
       p.un_scope()
@@ -795,8 +804,8 @@ class _Emitter:
       p.println('if (!row_mine)')
       p.do_scope()
       p.println('#pragma unroll')
-      p.println('for (int j = 0; j < %d; ++j) op%d[j] += a.stride[%d];' % (
-          self.VPT, node.output_index, s))
+      p.println('for (int j = 0; j < %d; ++j) op%d[j] += a.out_stride[%d][%d];'
+                % (self.VPT, node.output_index, node.output_index, s))
       p.un_scope()
       p.println('else')
     p.println('#pragma unroll')
@@ -926,8 +935,8 @@ class _Emitter:
       out = 'op%d[j]' % n
       if self.peel:
         out = 'orow'
-        p.println('%s* const orow = op%d[j] + pitch * %dll;' % (
-            node.c_type, n, phase))
+        p.println('%s* const orow = op%d[j] + opitch%d * %dll;' % (
+            node.c_type, n, n, phase))
       if self.steady:
         p.println('if (fast%d[j])' % n)
       else:
@@ -957,7 +966,7 @@ class _Emitter:
       p.println('for (int k = 0; k < %d; ++k)' % V)
       p.println('  o[k] = ((keep >> k) & 1u) ? static_cast<%s>(%s[k]%s) : '
                 '%s(0);' % (node.c_type, target, half, node.c_type))
-      p.println('if (own[j] == %du && a.vec_store)' % ((1 << V) - 1))
+      p.println('if (own[j] == %du && a.vec_store[%d])' % ((1 << V) - 1, n))
       p.do_scope()
       p.println('soda::st_pack_global<%s, %d>(%s, o);' % (node.c_type, V, out))
       p.un_scope()
@@ -969,7 +978,7 @@ class _Emitter:
       p.un_scope()
       p.un_scope()
       if not self.peel:
-        p.println('op%d[j] += a.stride[%d];' % (n, s))
+        p.println('op%d[j] += a.out_stride[%d][%d];' % (n, n, s))
     p.un_scope()
     p.un_scope()
 

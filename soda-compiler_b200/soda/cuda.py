@@ -167,6 +167,7 @@ class Library:
     lib = self._lib = ctypes.CDLL(path)
     c_int, c_void_p, c_char_p = ctypes.c_int, ctypes.c_void_p, ctypes.c_char_p
     i32p = ctypes.POINTER(ctypes.c_int32)
+    i64p = ctypes.POINTER(ctypes.c_int64)
     bufpp = ctypes.POINTER(ctypes.POINTER(BufferT))
     voidpp = ctypes.POINTER(c_void_p)
     for name, restype, argtypes in (
@@ -192,6 +193,8 @@ class Library:
         ('soda_cuda_run_batch', c_int, [bufpp, bufpp, bufpp, c_int]),
         ('soda_cuda_run_device_batch', c_int,
          [voidpp, voidpp, i32p, c_int, c_int, c_void_p]),
+        ('soda_cuda_run_device_strided', c_int,
+         [voidpp, i64p, voidpp, i64p, i32p, c_int, c_int, c_void_p]),
         ('soda_cuda_launch', c_int,
          [c_int, voidpp, voidpp, i32p, c_int, c_int, i32p, i32p, c_void_p]),
         ('soda_cuda_launch_chunked', c_int,
@@ -513,6 +516,128 @@ class Library:
     if code:
       raise CudaError('soda_cuda_run_device_batch(%s)' % self.app_name, code)
 
+  def run_device_strided(self, inputs, outputs, dims, batch, in_strides,
+                         out_strides, iterate=0, stream=None):
+    """``run_device_batch`` on arrays of any layout soda_cuda_run_device_strided
+    accepts (asynchronous).  ``in_strides`` / ``out_strides``: per tensor, its
+    element strides along dimensions 0 .. dim-1, then (batch > 1) the item
+    stride."""
+    code = self._lib.soda_cuda_run_device_strided(
+        self._pointers(inputs), self._strides(in_strides, batch),
+        self._pointers(outputs), self._strides(out_strides, batch),
+        (ctypes.c_int32 * 4)(*(list(dims) + [1] * (4 - len(dims)))), batch,
+        iterate, stream)
+    if code:
+      raise CudaError('soda_cuda_run_device_strided(%s)' % self.app_name,
+                      code)
+
+  def _strides(self, per_tensor, batch):
+    """5 int64 per tensor: strides of dimensions 0..3 (0 past the rank),
+    then the item stride (0 when not given)."""
+    flat = []
+    for strides in per_tensor:
+      strides = [int(v) for v in strides]
+      if len(strides) not in (self.dim, self.dim + 1):
+        raise ValueError('%d strides per tensor (and the item stride), got %d'
+                         % (self.dim, len(strides)))
+      item = strides[self.dim] if len(strides) > self.dim else 0
+      if batch > 1 and len(strides) == self.dim:
+        raise ValueError('a batch needs the item stride of every tensor')
+      flat += strides[:self.dim] + [0] * (4 - self.dim) + [item]
+    return (ctypes.c_int64 * len(flat))(*flat)
+
+  def run_strided(self, inputs, outputs=None, batched=False, iterate=0,
+                  stream=None):
+    """Run the program on torch CUDA tensors of any layout with unit stride
+    along the last axis and no two cells of a tensor at one address: views
+    (``x[..., 8:-8, 8:-8]``), rows of a pitched allocation, a channel of a
+    batch (``x[:, c]``), the interior of a larger output.  Nothing is copied.
+
+    Every tensor has shape ``(dims[n-1], .., dims[0])``, or with ``batched``
+    ``(B, dims[n-1], .., dims[0])``.  ``outputs``: tensors to fill, or None to
+    allocate contiguous ones.  Cells outside a view read as 0 (as outside a
+    grid) and nothing outside an output view is written.  Outputs must not
+    overlap the inputs or each other: this is not checked.  Runs on the
+    current torch stream of the inputs' device unless ``stream`` (a
+    cudaStream_t or torch stream) is given; asynchronous like the stream.
+    Param arrays are those of the last ``set_params``.  Host arrays go
+    through ``run`` / ``run_batch``."""
+    import torch
+    if len(inputs) != len(self.inputs):
+      raise ValueError('%s takes %d input(s)' % (self.app_name,
+                                                 len(self.inputs)))
+    if outputs is not None and len(outputs) != len(self.outputs):
+      raise ValueError('%s has %d output(s)' % (self.app_name,
+                                                len(self.outputs)))
+    rank = self.dim + (1 if batched else 0)
+    ins, extents = [], None
+    for array, (name, haoda_type) in zip(inputs, self.inputs):
+      got, strides = self._strided_view(array, haoda_type,
+                                        'input `%s`' % name, rank)
+      if extents is not None and got != extents:
+        raise ValueError('input `%s` has extent %s, expected %s' % (
+            name, got, extents))
+      extents = got
+      ins.append(strides)
+    device = inputs[0].device
+    if outputs is None:
+      outputs = [self._allocate_like(inputs[0], haoda_type, extents)
+                 for _, haoda_type in self.outputs]
+    outs = []
+    for array, (name, haoda_type) in zip(outputs, self.outputs):
+      got, strides = self._strided_view(array, haoda_type,
+                                        'output `%s`' % name, rank)
+      if got != extents:
+        raise ValueError('output `%s` has extent %s, expected %s' % (
+            name, got, extents))
+      outs.append(strides)
+    for array in list(inputs) + list(outputs):
+      if array.device != device:
+        raise ValueError('every tensor must be on %s, got %s' % (
+            device, array.device))
+    batch = extents[self.dim] if batched else 1
+    with torch.cuda.device(device):
+      if stream is None:
+        stream = torch.cuda.current_stream(device)
+      stream = getattr(stream, 'cuda_stream', stream)
+      self.run_device_strided(inputs, outputs, extents[:self.dim], batch,
+                              ins, outs, iterate, stream)
+    return list(outputs)
+
+  def _strided_view(self, array, haoda_type, what, rank):
+    """``(extents, element strides)`` of a torch CUDA tensor, dimension 0
+    first (items last); refuses what soda_cuda_run_device_strided would."""
+    import torch
+    if not isinstance(array, torch.Tensor) or not array.is_cuda:
+      raise TypeError('%s: run_strided takes torch CUDA tensors; host arrays '
+                      'go through run / run_batch' % what)
+    want = torch.from_numpy(np.empty(0, NUMPY_TYPES[haoda_type])).dtype
+    if array.dtype != want:
+      raise TypeError('%s must be %s, got %s' % (what, want, array.dtype))
+    if array.dim() != rank:
+      raise ValueError('%s must be %d-dimensional%s' % (
+          what, rank, ' (a leading batch dimension)' if rank > self.dim
+          else ''))
+    extents = tuple(reversed(array.shape))
+    strides = list(reversed(array.stride()))
+    if array.numel() == 0:
+      raise ValueError('%s is empty' % what)
+    # an axis of extent 1 has no stride that matters: give it the smallest
+    # the layout rule allows
+    for d in range(1, rank):
+      if extents[d] == 1:
+        strides[d] = strides[d - 1] * extents[d - 1]
+    if strides[0] != 1:
+      raise ValueError('%s must have stride 1 along its last axis, got %s' % (
+          what, tuple(array.stride())))
+    for d in range(1, rank):
+      if strides[d] < strides[d - 1] * extents[d - 1]:
+        raise ValueError(
+            '%s: layout not accepted (transposed, broadcast or overlapping): '
+            'axis strides %s for shape %s' % (
+                what, tuple(array.stride()), tuple(array.shape)))
+    return extents, strides
+
   def ipc_export(self, address):
     """``(handle bytes, offset)`` of the device allocation holding
     ``address``, for another process to map (see soda_cuda_ipc_export)."""
@@ -664,6 +789,28 @@ def run(stencil, arrays, params=None, devices=None, **kwargs):
     outputs = library.run(inputs, params=params, devices=devices)
     return {name: out for (name, _), out in zip(library.outputs, outputs)}
   return library.run(list(arrays), params=params, devices=devices)
+
+
+def run_strided(stencil, arrays, params=None, batched=False, iterate=0,
+                stream=None, **kwargs):
+  """Run ``stencil`` on torch CUDA tensors of any layout ``Library.run_strided``
+  accepts, without copying them; ``batched``: every tensor has a leading
+  batch dimension.  ``arrays`` and the result take the forms of ``run``;
+  ``params``, if given, are uploaded first (``Library.set_params``)."""
+  library = compile_stencil(stencil, **kwargs)
+  if isinstance(arrays, dict):
+    inputs = [arrays[name] for name, _ in library.inputs]
+    if params is None and library.params:
+      params = [arrays[name] for name, _, _ in library.params]
+  else:
+    inputs = list(arrays)
+  if params is not None:
+    library.set_params(params)
+  outputs = library.run_strided(inputs, batched=batched, iterate=iterate,
+                                stream=stream)
+  if isinstance(arrays, dict):
+    return {name: out for (name, _), out in zip(library.outputs, outputs)}
+  return outputs
 
 
 def run_batch(stencil, arrays, params=None, **kwargs):

@@ -118,6 +118,10 @@ def main():
       kind, name, iterate, _, options, _ = case
       jobs.append((str(name), test_batch_gpu._stencil(kind, name, iterate),
                    options))
+    import strided_programs
+    for kind, name, iterate, options in strided_programs.BUILDS:
+      jobs.append((str(name), strided_programs.stencil_of(kind, name, iterate),
+                   options))
     # the autotuner test times the planner's own choices, not tuned.json's
     import test_tune_gpu
     marks = [m for m in test_tune_gpu.test_tune_times_every_candidate
